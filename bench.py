@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the BASELINE.json metric: PAF post-processing images/sec at 368x432.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path (stages 1-5: bilinear x8 upsample materialising the
 operator-surface tensors, Gaussian smoothing, 3x3 NMS peak extraction, PAF line-integral scoring,
@@ -25,6 +25,8 @@ is one final result gather.  One JSON line is printed by rank 0.
                compiled into oracle/_ref/libpaf_ref.so) on ONE host core on a bounded sample
 
 --impl reference times that unmodified reference on all host cores (multiprocessing).
+--dump-outputs DIR writes what the headline loop returned in its last step to DIR/<name>.npy (dump_outputs); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -42,6 +44,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark only reads the tree it runs from (which may be read-only)
 
 METRIC = "postprocess images/sec at 368x432"
 UNIT = "images/s"
@@ -484,6 +487,48 @@ class Runner:
         self.torch.cuda.empty_cache()
 
 
+DUMP_MAT_POSITIONS = 256   # (y, x) positions per image sampled from heat_mat / paf_mat (2.3 GB per batch in full)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, R, nb):
+    """What the timed headline loop handed its caller in its last step, as DIR/<name>.npy (float32 / float64), so that two
+    builds can be compared output for output.  Every context still holds the batch it ran last, so the last
+    min(contexts, batches per step) batches of the step are read back, as many of them as fit DUMP_LIMIT_BYTES: their
+    result tables (rows past num_humans / n_peaks zeroed) and the operator-surface tensors at a fixed, seeded sample of
+    positions.  Dumped batches are stacked along a leading axis, the oldest first."""
+    torch = R.torch
+    pp0 = R.pps[0]
+    per_batch = R.n * (8 * (3 + 19) + 4 * (20 * pp0.max_humans + 4 * pp0.max_peaks + 57 * DUMP_MAT_POSITIONS))
+    fit = (DUMP_LIMIT_BYTES - 16 * DUMP_MAT_POSITIONS) // per_batch
+    batches = range(nb - max(1, min(BATCHES_PER_STEP, R.mat_nctx, nb, fit)), nb)
+    rng = np.random.default_rng(0)
+    ys = torch.from_numpy(rng.integers(0, 8 * R.h, DUMP_MAT_POSITIONS)).to(R.dev)
+    xs = torch.from_numpy(rng.integers(0, 8 * R.w, DUMP_MAT_POSITIONS)).to(R.dev)
+    cols = {k: [] for k in ("num_humans", "n_peaks", "overflow", "subset", "peaks", "part_off", "heat_mat_sample", "paf_mat_sample")}
+    for i in batches:
+        pp = R.pps[i % R.mat_nctx]
+        res = pp.results(with_peaks=True, raise_on_overflow=False)
+        subset = res["subset"].copy()
+        peaks = np.stack([res["peaks"][f].astype(np.float32) for f in ("x", "y", "score", "id")], axis=-1)
+        for j in range(len(subset)):
+            subset[j, int(res["num_humans"][j]):] = 0
+            peaks[j, int(res["n_peaks"][j]):] = 0
+        for k in ("num_humans", "n_peaks", "overflow", "part_off"):
+            cols[k].append(res[k].astype(np.float64))
+        cols["subset"].append(subset)
+        cols["peaks"].append(peaks)
+        cols["heat_mat_sample"].append(pp.heat_mat[:, ys, xs, :].cpu().numpy())
+        cols["paf_mat_sample"].append(pp.paf_mat[:, ys, xs, :].cpu().numpy())
+    arrays = {k: np.stack(v) for k, v in cols.items()}
+    arrays["mat_sample_yx"] = np.stack([ys.cpu().numpy(), xs.cpu().numpy()], axis=1).astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"dump of {total} bytes exceeds {DUMP_LIMIT_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 FRONTEND_KERNELS = {("dense", True): ["dense_frontend_kernel<mat>"], ("dense", False): ["dense_plane_kernel"],
                     ("reference", False): ["ref_scan_kernel", "ref_refine_kernel"]}
 STAGE_BOUNDS = {
@@ -606,6 +651,8 @@ def run_ours(args, rank, local_rank, world):
     launches, graph_batches = l1 - l0, g1 - g0
     res = R.pps[(nb - 1) % N_CTX].results()
     total_humans = int(res["num_humans"].sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, R, nb)
     iso_ms = R.isolated_stage_ms("dense", True)
     c2_check = R.oracle_check("dense", True) if rank == 0 else None
 
@@ -900,6 +947,7 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the configs[2..4] context legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed loop's last step to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -915,6 +963,8 @@ def main():
                "--steps", str(args.steps), "--warmup", str(args.warmup)]
         if args.headline_only:
             cmd.append("--headline-only")
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)]
         raise SystemExit(subprocess.call(cmd))
     run_ours(args, rank, local_rank, world)
 

@@ -3,6 +3,7 @@ without a GPU, and the product never routes through the oracle."""
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 
 import numpy as np
@@ -43,7 +44,11 @@ def test_python_binding_covers_the_header():
 
 
 def test_sass_is_sm_100a_only():
-    out = subprocess.run(["cuobjdump", "-lelf", SO], capture_output=True, text=True).stdout
+    # next to the nvcc torch_ekpose_b200/csrc/Makefile builds with (NVCC ?= /usr/local/cuda/bin/nvcc), on PATH or not
+    nvcc = shutil.which(os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc"))
+    assert nvcc, "the nvcc the library was built with is not found"
+    cuobjdump = os.path.join(os.path.dirname(nvcc), "cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", SO], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 
