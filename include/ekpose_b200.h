@@ -48,6 +48,11 @@ typedef enum ekp_status {
 
 typedef enum ekp_layout { EKP_LAYOUT_NCHW = 0, EKP_LAYOUT_NHWC = 1 } ekp_layout;
 
+/* element type of the heat / PAF inputs of the *_typed entry points.  16-bit maps (what the network returns under
+ * torch.autocast) are widened to float32 on the device (exact: every finite value, +-0, subnormals and +-inf; a NaN
+ * stays a NaN) and then take the float32 path, so the results equal those of the float32 maps x.float(). */
+typedef enum ekp_dtype { EKP_DTYPE_F32 = 0, EKP_DTYPE_BF16 = 1, EKP_DTYPE_F16 = 2 } ekp_dtype;
+
 /* which peak front-end runs as stages 1-3 */
 typedef enum ekp_frontend {
     EKP_FRONTEND_DENSE = 0,     /* bilinear x8 -> Gaussian sigma 3 -> 3x3 max NMS (BASELINE.json north_star) */
@@ -124,6 +129,19 @@ int ekp_postprocess(ekp_ctx *ctx, const float *heat, const float *paf, int n, in
 int ekp_postprocess_host(ekp_ctx *ctx, const float *heat_host, const float *paf_host, int n, int h, int w,
                          int layout, float thr_heat, int frontend, int materialize, void *stream);
 
+/* ekp_postprocess / ekp_postprocess_host for inputs of element type `dtype` (ekp_dtype).  EKP_DTYPE_F32 is exactly the
+ * two calls above.  EKP_DTYPE_BF16 / EKP_DTYPE_F16: heat / paf hold 16-bit values in the same shapes and layouts and
+ * need 2-byte alignment; one kernel widens both to float32 into a context-owned device block (allocated on first use,
+ * max_batch x max_h x max_w x 57 floats), then the float32 kernels run on it.  heat_mat / paf_mat stay float32.
+ * The host variant copies the 16-bit buffers (half the bytes of float32) into a second context-owned 16-bit device
+ * block first: ONE copy when heat is directly followed by paf in host memory, as for float32.  The widening kernel
+ * counts in ekp_kernel_launches, its time in stage [0] of ekp_stage_times, and it is part of the batch's CUDA graph.
+ * An unknown dtype or a 16-bit pointer that is not 2-byte aligned returns EKP_ERR_ARG. */
+int ekp_postprocess_typed(ekp_ctx *ctx, const void *heat, const void *paf, int dtype, int n, int h, int w, int layout,
+                          float thr_heat, int frontend, float *heat_mat, float *paf_mat, void *stream);
+int ekp_postprocess_host_typed(ekp_ctx *ctx, const void *heat_host, const void *paf_host, int dtype, int n, int h,
+                               int w, int layout, float thr_heat, int frontend, int materialize, void *stream);
+
 /* Stages 4-5 only, DEVICE inputs: per image a peak list in the reference's format
  * float32 [n, peaks_stride, 5] rows (x, y, score, <ignored>, part) (pafprocess.cpp:26-36) with
  * n_peaks[i] valid rows, and the full-resolution PAF tensor float32 [n, H, W, C] the reference
@@ -177,7 +195,8 @@ int ekp_preprocess(ekp_ctx *ctx, const unsigned char *frames, int n, int src_h, 
 
 /* Per-stage device timing for the benchmark.  When enabled, CUDA events are recorded on the work
  * stream around each stage of every run (a ring of the last 64 runs).  ekp_stage_times waits for
- * the stream and returns the mean milliseconds of: [0] stages 1-3 (front-end kernel(s)),
+ * the stream and returns the mean milliseconds of: [0] stages 1-3 (front-end kernel(s); for 16-bit inputs
+ * also the widening kernel of the *_typed entry points),
  * [1] peak sort, [2] stage 4 + sort/greedy (paf_connect), [3] assembly; *runs = runs averaged. */
 int ekp_set_timing(ekp_ctx *ctx, int enable);
 int ekp_stage_times(ekp_ctx *ctx, float *ms, int *runs);
@@ -196,6 +215,9 @@ long long ekp_graph_launches(const ekp_ctx *ctx);  /* batches of those that were
  * PAF tensor in ONE such block the library moves both with a single copy.  write_combined != 0 asks for
  * write-combined memory (CPU writes only, sequential). */
 int ekp_host_alloc(void **out, size_t bytes, int write_combined);
+/* Releasing a block also retires the CUDA graphs of host-entry batches captured before it (they are captured again on
+ * their next submission), so a new block that comes back at the address of a released one is never read through a
+ * graph of the old one. */
 int ekp_host_free(void *p);
 
 /* ---- the reference operator surface (lib/pafprocess/pafprocess.h:53-59) ------------------

@@ -15,6 +15,7 @@ SO_PATH = os.environ.get("EKPOSE_B200_SO") or os.path.join(HERE, "libekpose_b200
 
 NUM_PART, NUM_LIMB, HEAT_CH, PAF_CH, UP, SUBSET_COLS = 18, 19, 19, 38, 8, 20
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2
 FRONTEND_DENSE, FRONTEND_REFERENCE, FRONTEND_REFERENCE_COARSE, FRONTEND_REFERENCE_GAUSS = 0, 1, 2, 3
 OK, ERR_ARG, ERR_CUDA, ERR_CAPACITY, ERR_STATE = 0, -1, -2, -3, -4
 OVF_PEAKS, OVF_PART, OVF_CANDIDATES, OVF_HUMANS, OVF_BADPEAK = 1, 2, 4, 8, 16
@@ -46,6 +47,8 @@ SIGNATURES = {
     "ekp_version": (C.c_char_p, []),
     "ekp_postprocess": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp]),
     "ekp_postprocess_host": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _i, _vp]),
+    "ekp_postprocess_typed": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp]),
+    "ekp_postprocess_host_typed": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _i, _vp]),
     "ekp_process_paf_dev": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "ekp_results": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "ekp_results_humans": (_i, [_vp, _vp, _vp, _vp, _vp]),

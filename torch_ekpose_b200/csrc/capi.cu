@@ -49,6 +49,8 @@ cudaError_t launch_debug_std_sort(float* scores, unsigned* tags, int n, unsigned
 cudaError_t launch_preprocess(const unsigned char* src, float* out, const int* xofs, const short* ialpha, const int* yofs,
                               const short* ibeta, int n, int sh, int sw, int rh, int rw, int ph, int pw, int mode,
                               cudaStream_t stream);
+cudaError_t launch_widen(const void* heat16, const void* paf16, size_t n_heat, size_t n_paf, int dtype, float* heat, float* paf,
+                         cudaStream_t stream);
 }  // namespace ekp
 
 using namespace ekp;
@@ -152,20 +154,27 @@ extern "C" int ekp_scipy_gauss3_weights(double* out13) {
 // ---- context -----------------------------------------------------------------------------------
 // arguments of one batch submission (also the key of its CUDA graph)
 struct PostArgs {
-    const float *heat, *paf;            // device inputs
-    const float *heat_host, *paf_host;  // host inputs to copy in first (nullptr: the device pointers are the caller's)
+    const float *heat, *paf;            // float32 device inputs of stages 1-3
+    const void *heat_host, *paf_host;   // host inputs to copy in first (nullptr: the device pointers are the caller's)
     size_t h2d_heat_bytes, h2d_paf_bytes;
+    const void *heat16, *paf16;         // 16-bit device inputs widened into heat / paf first (EKP_DTYPE_BF16 / EKP_DTYPE_F16)
+    int dtype;
     int n, h, w, layout, frontend;
     float thr;
     float *heat_mat, *paf_mat;
 };
 static bool same_args(const PostArgs& a, const PostArgs& b) {
-    return a.heat == b.heat && a.paf == b.paf && a.heat_host == b.heat_host && a.paf_host == b.paf_host && a.n == b.n && a.h == b.h &&
+    return a.heat == b.heat && a.paf == b.paf && a.heat_host == b.heat_host && a.paf_host == b.paf_host && a.heat16 == b.heat16 &&
+           a.paf16 == b.paf16 && a.dtype == b.dtype && a.n == b.n && a.h == b.h &&
            a.w == b.w && a.layout == b.layout && a.frontend == b.frontend && memcmp(&a.thr, &b.thr, sizeof(float)) == 0 &&
            a.heat_mat == b.heat_mat && a.paf_mat == b.paf_mat;
 }
 
-struct GraphEntry { PostArgs key; cudaGraphExec_t exec; int kernels; unsigned long long stamp; };
+// host_epoch: g_host_frees when a graph with host inputs was captured.  Its copy nodes refer to the pinned allocation that
+// held them; once any block is released by ekp_host_free a new block may come back at the same address, so such graphs
+// are not replayed across an ekp_host_free (they would copy from the released allocation).
+struct GraphEntry { PostArgs key; cudaGraphExec_t exec; int kernels; unsigned long long stamp, host_epoch; };
+static std::atomic<unsigned long long> g_host_frees{0};
 
 struct ekp_ctx {
     int device = 0, max_batch = 0, max_h = 0, max_w = 0, max_peaks = 0, max_humans = 0;
@@ -182,6 +191,8 @@ struct ekp_ctx {
     unsigned char* records = nullptr;  // [max_batch] packed result records (ResultLayout)
     ResultLayout lay = {};
     float* in_block = nullptr;      // staging for the host-buffer entry point: [heat | paf] of one batch, contiguous
+                                    // (also where 16-bit inputs are widened to)
+    void* in_block16 = nullptr;     // 16-bit [heat | paf] staging of the host-buffer entry point (lazily, half of in_block)
     float* mat_heat = nullptr;      // context-owned operator-surface tensors (host entry, lazily)
     float* mat_paf = nullptr;
     size_t mat_images = 0, mat_hw = 0;
@@ -223,7 +234,7 @@ static int ctx_free(ekp_ctx* c) {
     if (!c) return EKP_OK;
     cudaSetDevice(c->device);
     void* dev[] = {c->raw, c->raw_count, c->line, c->part_off, c->n_peaks, c->conns, c->n_conns, c->records,
-                   c->in_block, c->mat_heat, c->mat_paf, c->ax, c->ay, c->cubic, c->gauss, c->prep_tab};
+                   c->in_block, c->in_block16, c->mat_heat, c->mat_paf, c->ax, c->ay, c->cubic, c->gauss, c->prep_tab};
     for (void* p : dev) if (p) cudaFree(p);
     void* host[] = {c->h_records, c->h_line};
     for (void* p : host) if (p) cudaFreeHost(p);
@@ -337,6 +348,7 @@ extern "C" int ekp_host_alloc(void** out, size_t bytes, int write_combined) {
 }
 extern "C" int ekp_host_free(void* p) {
     if (p) CU(cudaFreeHost(p));
+    g_host_frees.fetch_add(1, std::memory_order_acq_rel);
     return EKP_OK;
 }
 
@@ -419,22 +431,30 @@ static int run_back_half(ekp_ctx* c, int n, int id_from_key, const PafSource& pa
 // device-to-host copy of the result records.  Issued eagerly or into a stream capture; returns the kernels launched.
 static int enqueue_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st, int* kernels) {
     int k = 0;
+    const bool wide = a.dtype == EKP_DTYPE_F32;
     if (a.heat_host) {
+        // the copies land where the kernels read: the float32 block, or the 16-bit block that is widened into it below
+        char* dh = static_cast<char*>(const_cast<void*>(wide ? static_cast<const void*>(a.heat) : a.heat16));
+        char* dp = static_cast<char*>(const_cast<void*>(wide ? static_cast<const void*>(a.paf) : a.paf16));
         // one copy when the caller's two tensors are adjacent in host memory (one pinned block: heat, then paf), else two
-        if (reinterpret_cast<const char*>(a.heat_host) + a.h2d_heat_bytes == reinterpret_cast<const char*>(a.paf_host) &&
-            reinterpret_cast<const char*>(a.heat) + a.h2d_heat_bytes == reinterpret_cast<const char*>(a.paf)) {
-            CU(cudaMemcpyAsync(const_cast<float*>(a.heat), a.heat_host, a.h2d_heat_bytes + a.h2d_paf_bytes, cudaMemcpyHostToDevice, st));
+        if (static_cast<const char*>(a.heat_host) + a.h2d_heat_bytes == static_cast<const char*>(a.paf_host) && dh + a.h2d_heat_bytes == dp) {
+            CU(cudaMemcpyAsync(dh, a.heat_host, a.h2d_heat_bytes + a.h2d_paf_bytes, cudaMemcpyHostToDevice, st));
         } else {
-            CU(cudaMemcpyAsync(const_cast<float*>(a.heat), a.heat_host, a.h2d_heat_bytes, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(const_cast<float*>(a.paf), a.paf_host, a.h2d_paf_bytes, cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpyAsync(dh, a.heat_host, a.h2d_heat_bytes, cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpyAsync(dp, a.paf_host, a.h2d_paf_bytes, cudaMemcpyHostToDevice, st));
         }
     }
     CU(cudaMemsetAsync(c->raw_count, 0, sizeof(int) * 2 * (size_t) c->max_batch, st));
+    mark(c, 0, st);
+    if (!wide) {
+        const size_t px = (size_t) a.n * a.h * a.w;
+        CU(launch_widen(a.heat16, a.paf16, px * EKP_HEAT_CH, px * EKP_PAF_CH, a.dtype, const_cast<float*>(a.heat), const_cast<float*>(a.paf), st));
+        k += 1;
+    }
     PafSource src;
     src.layout = a.layout; src.H = 8 * a.h; src.W = 8 * a.w; src.C = EKP_PAF_CH; src.h = a.h; src.w = a.w;
     src.pair_base = nullptr; src.ids_are_rows = 1;
     if (a.frontend == EKP_FRONTEND_DENSE) {
-        mark(c, 0, st);
         DenseParams p;
         p.heat = a.heat; p.paf = a.paf; p.n = a.n; p.h = a.h; p.w = a.w; p.layout = a.layout; p.thr = a.thr;
         p.ax = c->ax; p.ay = c->ay; p.heat_mat = a.heat_mat; p.paf_mat = a.paf_mat; p.smooth_out = nullptr;
@@ -449,7 +469,6 @@ static int enqueue_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st, int* ke
         if (a.paf_mat && from_mat) { src.ptr = a.paf_mat; src.mode = PAF_FULL_HWC; }
         else { src.ptr = a.paf; src.mode = PAF_LO_BILINEAR; }
     } else {
-        mark(c, 0, st);
         RefParams p;
         p.heat = a.heat; p.n = a.n; p.h = a.h; p.w = a.w; p.layout = a.layout; p.thr = a.thr;
         p.raw = c->raw; p.raw_count = c->raw_count; p.raw_cap = c->max_peaks; p.cubic = c->cubic;
@@ -487,7 +506,14 @@ static int submit_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
     } else {
         std::vector<GraphEntry>& G = *c->graphs;
         GraphEntry* hit = nullptr;
-        for (GraphEntry& e : G) if (same_args(e.key, a)) hit = &e;
+        const unsigned long long epoch = a.heat_host ? g_host_frees.load(std::memory_order_acquire) : 0;
+        for (size_t i = 0; i < G.size(); i++) {
+            if (!same_args(G[i].key, a)) continue;
+            if (G[i].host_epoch == epoch) { hit = &G[i]; break; }
+            cudaGraphExecDestroy(G[i].exec);  // captured before a host block was released: capture again
+            G.erase(G.begin() + (long) i);
+            break;
+        }
         if (!hit) {
             if (!c->cap_stream) CU(cudaStreamCreateWithFlags(&c->cap_stream, cudaStreamNonBlocking));
             cudaGraph_t graph = nullptr;
@@ -508,7 +534,7 @@ static int submit_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
                 cudaGraphExecDestroy(G[lru].exec);
                 G.erase(G.begin() + (long) lru);
             }
-            G.push_back(GraphEntry{a, exec, kernels, 0});
+            G.push_back(GraphEntry{a, exec, kernels, 0, epoch});
             hit = &G.back();
         }
         hit->stamp = ++c->graph_clock;
@@ -528,16 +554,33 @@ static int check_post_args(const ekp_ctx* c, int n, int h, int w, int layout, in
     return EKP_OK;
 }
 
-extern "C" int ekp_postprocess(ekp_ctx* c, const float* heat, const float* paf, int n, int h, int w, int layout,
-                               float thr_heat, int frontend, float* heat_mat, float* paf_mat, void* stream) {
-    int rc = check_post_args(c, n, h, w, layout, frontend, "ekp_postprocess");
+static int check_dtype(int dtype, const void* heat, const void* paf, const char* who) {
+    if (dtype != EKP_DTYPE_F32 && dtype != EKP_DTYPE_BF16 && dtype != EKP_DTYPE_F16)
+        return fail(EKP_ERR_ARG, "%s: dtype %d (EKP_DTYPE_F32 0, EKP_DTYPE_BF16 1, EKP_DTYPE_F16 2)", who, dtype);
+    if (dtype != EKP_DTYPE_F32 && ((reinterpret_cast<uintptr_t>(heat) | reinterpret_cast<uintptr_t>(paf)) & 1u))
+        return fail(EKP_ERR_ARG, "%s: 16-bit heat / paf must be 2-byte aligned", who);
+    return EKP_OK;
+}
+
+// the context's float32 input block [heat | paf] (host entry: the copy target; 16-bit inputs: the widening target)
+static int ensure_in_block(ekp_ctx* c) {
+    if (!c->in_block)  // ONE staging block: heat, directly followed by paf (so adjacent host tensors arrive with one copy)
+        CU(cudaMalloc((void**) &c->in_block, sizeof(float) * (size_t) c->max_batch * c->max_h * c->max_w * (EKP_HEAT_CH + EKP_PAF_CH)));
+    return EKP_OK;
+}
+
+static int postprocess_dev(ekp_ctx* c, const void* heat, const void* paf, int dtype, int n, int h, int w, int layout, float thr_heat,
+                           int frontend, float* heat_mat, float* paf_mat, void* stream, const char* who) {
+    int rc = check_post_args(c, n, h, w, layout, frontend, who);
     if (rc) return rc;
-    if (!heat || !paf) return fail(EKP_ERR_ARG, "ekp_postprocess: NULL input");
-    if (heat_mat && !paf_mat) return fail(EKP_ERR_ARG, "ekp_postprocess: heat_mat without paf_mat");
+    if (!heat || !paf) return fail(EKP_ERR_ARG, "%s: NULL input", who);
+    rc = check_dtype(dtype, heat, paf, who);
+    if (rc) return rc;
+    if (heat_mat && !paf_mat) return fail(EKP_ERR_ARG, "%s: heat_mat without paf_mat", who);
     if ((reinterpret_cast<uintptr_t>(heat_mat) | reinterpret_cast<uintptr_t>(paf_mat)) & 15u)
-        return fail(EKP_ERR_ARG, "ekp_postprocess: heat_mat / paf_mat must be 16-byte aligned (they are written with 16-byte bulk copies)");
-    if ((reinterpret_cast<uintptr_t>(heat) | reinterpret_cast<uintptr_t>(paf)) & 3u)
-        return fail(EKP_ERR_ARG, "ekp_postprocess: heat / paf must be 4-byte aligned");
+        return fail(EKP_ERR_ARG, "%s: heat_mat / paf_mat must be 16-byte aligned (they are written with 16-byte bulk copies)", who);
+    if (dtype == EKP_DTYPE_F32 && ((reinterpret_cast<uintptr_t>(heat) | reinterpret_cast<uintptr_t>(paf)) & 3u))
+        return fail(EKP_ERR_ARG, "%s: heat / paf must be 4-byte aligned", who);
     cudaStream_t st = (cudaStream_t) stream;
     CU(cudaSetDevice(c->device));
     if (frontend == EKP_FRONTEND_DENSE) {
@@ -545,20 +588,33 @@ extern "C" int ekp_postprocess(ekp_ctx* c, const float* heat, const float* paf, 
         if (rc) return rc;
     }
     PostArgs a = {};
-    a.heat = heat; a.paf = paf; a.n = n; a.h = h; a.w = w; a.layout = layout; a.frontend = frontend; a.thr = thr_heat;
+    a.dtype = dtype;
+    if (dtype == EKP_DTYPE_F32) {
+        a.heat = static_cast<const float*>(heat); a.paf = static_cast<const float*>(paf);
+    } else {
+        rc = ensure_in_block(c);
+        if (rc) return rc;
+        a.heat16 = heat; a.paf16 = paf;
+        a.heat = c->in_block; a.paf = c->in_block + (size_t) n * h * w * EKP_HEAT_CH;
+    }
+    a.n = n; a.h = h; a.w = w; a.layout = layout; a.frontend = frontend; a.thr = thr_heat;
     a.heat_mat = heat_mat; a.paf_mat = paf_mat;
     return submit_batch(c, a, st);
 }
 
-extern "C" int ekp_postprocess_host(ekp_ctx* c, const float* heat_host, const float* paf_host, int n, int h, int w,
-                                    int layout, float thr_heat, int frontend, int materialize, void* stream) {
-    int rc = check_post_args(c, n, h, w, layout, frontend, "ekp_postprocess_host");
+static int postprocess_host(ekp_ctx* c, const void* heat_host, const void* paf_host, int dtype, int n, int h, int w, int layout,
+                            float thr_heat, int frontend, int materialize, void* stream, const char* who) {
+    int rc = check_post_args(c, n, h, w, layout, frontend, who);
     if (rc) return rc;
-    if (!heat_host || !paf_host) return fail(EKP_ERR_ARG, "ekp_postprocess_host: NULL input");
+    if (!heat_host || !paf_host) return fail(EKP_ERR_ARG, "%s: NULL input", who);
+    rc = check_dtype(dtype, heat_host, paf_host, who);
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t) stream;
     CU(cudaSetDevice(c->device));
-    if (!c->in_block)  // ONE staging block: heat, directly followed by paf (so adjacent host tensors arrive with one copy)
-        CU(cudaMalloc((void**) &c->in_block, sizeof(float) * (size_t) c->max_batch * c->max_h * c->max_w * (EKP_HEAT_CH + EKP_PAF_CH)));
+    rc = ensure_in_block(c);
+    if (rc) return rc;
+    if (dtype != EKP_DTYPE_F32 && !c->in_block16)  // the 16-bit copy target, laid out like in_block
+        CU(cudaMalloc(&c->in_block16, 2 * (size_t) c->max_batch * c->max_h * c->max_w * (EKP_HEAT_CH + EKP_PAF_CH)));
     const size_t hw = (size_t) h * w;
     float *hm = nullptr, *pm = nullptr;
     if (materialize) {
@@ -581,13 +637,37 @@ extern "C" int ekp_postprocess_host(ekp_ctx* c, const float* heat_host, const fl
         rc = ensure_tables(c, h, w, st);
         if (rc) return rc;
     }
+    const size_t elem = dtype == EKP_DTYPE_F32 ? sizeof(float) : 2;
     PostArgs a = {};
-    a.heat_host = heat_host; a.paf_host = paf_host;
-    a.h2d_heat_bytes = sizeof(float) * (size_t) n * hw * EKP_HEAT_CH;
-    a.h2d_paf_bytes = sizeof(float) * (size_t) n * hw * EKP_PAF_CH;
+    a.heat_host = heat_host; a.paf_host = paf_host; a.dtype = dtype;
+    a.h2d_heat_bytes = elem * (size_t) n * hw * EKP_HEAT_CH;
+    a.h2d_paf_bytes = elem * (size_t) n * hw * EKP_PAF_CH;
     a.heat = c->in_block; a.paf = c->in_block + (size_t) n * hw * EKP_HEAT_CH;
+    if (dtype != EKP_DTYPE_F32) { a.heat16 = c->in_block16; a.paf16 = static_cast<char*>(c->in_block16) + a.h2d_heat_bytes; }
     a.n = n; a.h = h; a.w = w; a.layout = layout; a.frontend = frontend; a.thr = thr_heat; a.heat_mat = hm; a.paf_mat = pm;
     return submit_batch(c, a, st);
+}
+
+extern "C" int ekp_postprocess(ekp_ctx* c, const float* heat, const float* paf, int n, int h, int w, int layout,
+                               float thr_heat, int frontend, float* heat_mat, float* paf_mat, void* stream) {
+    return postprocess_dev(c, heat, paf, EKP_DTYPE_F32, n, h, w, layout, thr_heat, frontend, heat_mat, paf_mat, stream, "ekp_postprocess");
+}
+
+extern "C" int ekp_postprocess_typed(ekp_ctx* c, const void* heat, const void* paf, int dtype, int n, int h, int w, int layout,
+                                     float thr_heat, int frontend, float* heat_mat, float* paf_mat, void* stream) {
+    return postprocess_dev(c, heat, paf, dtype, n, h, w, layout, thr_heat, frontend, heat_mat, paf_mat, stream, "ekp_postprocess_typed");
+}
+
+extern "C" int ekp_postprocess_host(ekp_ctx* c, const float* heat_host, const float* paf_host, int n, int h, int w,
+                                    int layout, float thr_heat, int frontend, int materialize, void* stream) {
+    return postprocess_host(c, heat_host, paf_host, EKP_DTYPE_F32, n, h, w, layout, thr_heat, frontend, materialize, stream,
+                            "ekp_postprocess_host");
+}
+
+extern "C" int ekp_postprocess_host_typed(ekp_ctx* c, const void* heat_host, const void* paf_host, int dtype, int n, int h, int w,
+                                          int layout, float thr_heat, int frontend, int materialize, void* stream) {
+    return postprocess_host(c, heat_host, paf_host, dtype, n, h, w, layout, thr_heat, frontend, materialize, stream,
+                            "ekp_postprocess_host_typed");
 }
 
 extern "C" int ekp_process_paf_dev(ekp_ctx* c, const float* peaks, const int* n_peaks, int peaks_stride, int n, int h1,

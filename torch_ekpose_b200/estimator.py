@@ -63,7 +63,8 @@ def get_outputs_batched(images, model, preprocess: str, device):
 def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, frontend: str = "reference",
                  thr: float = 0.15) -> List[list]:
     """images -> per-image list[Human]: GPU preprocessing, one forward pass, post-processing on the same GPU
-    (the network's outputs never leave the device).  ``frontend='reference'`` gives the reference's people."""
+    (the network's outputs never leave the device, and 16-bit outputs of a model under torch.autocast are taken as
+    they are).  ``frontend='reference'`` gives the reference's people."""
     pafs, heats, _ = get_outputs_batched(images, model, preprocess, device)
     n, _, h, w = heats.shape
     idx = heats.device.index
@@ -72,7 +73,7 @@ def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, f
     if pp is None:
         pp = _pp_cache[key] = PostProcessor(device=idx, max_batch=n, max_h=h, max_w=w, max_peaks=2048, max_humans=128)
     _last_pp[0] = pp
-    pp.run(heats.float(), pafs.float(), layout="nchw", frontend=frontend, thr=thr)
+    pp.run(heats, pafs, layout="nchw", frontend=frontend, thr=thr)   # bf16 / fp16 under autocast: widened on the device
     return pp.humans()
 
 

@@ -42,12 +42,22 @@ def _is_tensor(x) -> bool:
     return torch is not None and isinstance(x, torch.Tensor)
 
 
+def _dtype16(heat, paf) -> int:
+    """The library's 16-bit dtype code when heat and paf are both bf16 / fp16 tensors, or both NumPy float16 arrays, of
+    the same dtype; else 0 (EKP_DTYPE_F32: the float32 path, with a conversion for anything that is not float32)."""
+    if _is_tensor(heat) and _is_tensor(paf) and heat.dtype == paf.dtype:
+        return {torch.bfloat16: _lib.DTYPE_BF16, torch.float16: _lib.DTYPE_F16}.get(heat.dtype, 0)
+    if isinstance(heat, np.ndarray) and isinstance(paf, np.ndarray) and heat.dtype == paf.dtype == np.float16:
+        return _lib.DTYPE_F16
+    return 0
+
+
 class PostProcessor:
     """A libekpose_b200 context: stages 1-5 for batches of up to ``max_batch`` images.
 
     ``run`` is asynchronous on the current CUDA stream of ``device``; ``results`` / ``humans`` /
-    ``peaks`` wait for it.  Inputs are float32 stride-8 maps, ``heat`` with 19 and ``paf`` with 38
-    channels, layout ``'nchw'`` (lib/network/vgg2016.py:105) or ``'nhwc'``
+    ``peaks`` wait for it.  Inputs are float32, bfloat16 or float16 stride-8 maps, ``heat`` with 19 and
+    ``paf`` with 38 channels, layout ``'nchw'`` (lib/network/vgg2016.py:105) or ``'nhwc'``
     (lib/evaluate/estimator.py:85-86).
     """
 
@@ -107,6 +117,10 @@ class PostProcessor:
             materialize: bool = False, stream=None) -> None:
         """Submit one batch (n <= max_batch).  CUDA tensors take the device entry point; NumPy
         arrays / CPU tensors take the host entry point (H2D copies on the same stream).
+        heat and paf of the same 16-bit dtype (torch.bfloat16 / torch.float16 tensors, NumPy float16 arrays: what a
+        network returns under torch.autocast) are handed over as they are and widened to float32 on the device, which
+        gives exactly the results of their .float(); on the host entry only half the bytes cross the bus.  Any other
+        dtype (mixed, float64, ...) is converted to float32 here.
         frontend: 'reference' (default: the reference's own stride-8 NMS + bicubic refinement, i.e. the people
         paf_to_pose_cpp returns), 'dense' (the north_star formulation), 'reference_coarse' (NMS(bool_refine_center=False))
         or 'reference_gauss' (NMS(bool_gaussian_filt=True))."""
@@ -120,8 +134,11 @@ class PostProcessor:
                 raise ValueError("heat and paf must live on the same device")
             if heat.device.index != self.device:
                 raise ValueError(f"tensors are on cuda:{heat.device.index}, context on cuda:{self.device}")
-            heat = heat.contiguous().float()
-            paf = paf.contiguous().float()
+            dtype = _dtype16(heat, paf)
+            if dtype:
+                heat, paf = heat.contiguous(), paf.contiguous()
+            else:
+                heat, paf = heat.contiguous().float(), paf.contiguous().float()
             hm = pm = None
             if materialize:
                 H, W = 8 * h, 8 * w
@@ -129,19 +146,21 @@ class PostProcessor:
                     self.heat_mat = torch.empty((n, H, W, _lib.HEAT_CH), dtype=torch.float32, device=heat.device)
                     self.paf_mat = torch.empty((n, H, W, _lib.PAF_CH), dtype=torch.float32, device=heat.device)
                 hm, pm = self.heat_mat.data_ptr(), self.paf_mat.data_ptr()
-            rc = _lib.lib.ekp_postprocess(self._ctx, heat.data_ptr(), paf.data_ptr(), n, h, w, _LAYOUTS[layout], thr,
-                                          _FRONTENDS[frontend], hm, pm, st)
+            rc = _lib.lib.ekp_postprocess_typed(self._ctx, heat.data_ptr(), paf.data_ptr(), dtype, n, h, w, _LAYOUTS[layout],
+                                                thr, _FRONTENDS[frontend], hm, pm, st)
             self._keep = (heat, paf)
         else:
+            dtype = _dtype16(heat, paf)
             if _is_tensor(heat):
-                heat_p, paf_p = heat.contiguous().float(), paf.contiguous().float()
+                heat_p, paf_p = (heat.contiguous(), paf.contiguous()) if dtype else (heat.contiguous().float(), paf.contiguous().float())
                 ptrs = (heat_p.data_ptr(), paf_p.data_ptr())
             else:
-                heat_p = np.ascontiguousarray(heat, np.float32)
-                paf_p = np.ascontiguousarray(paf, np.float32)
+                want = np.float16 if dtype else np.float32
+                heat_p = np.ascontiguousarray(heat, want)
+                paf_p = np.ascontiguousarray(paf, want)
                 ptrs = (heat_p.ctypes.data, paf_p.ctypes.data)
-            rc = _lib.lib.ekp_postprocess_host(self._ctx, ptrs[0], ptrs[1], n, h, w, _LAYOUTS[layout], thr,
-                                               _FRONTENDS[frontend], int(bool(materialize)), st)
+            rc = _lib.lib.ekp_postprocess_host_typed(self._ctx, ptrs[0], ptrs[1], dtype, n, h, w, _LAYOUTS[layout], thr,
+                                                     _FRONTENDS[frontend], int(bool(materialize)), st)
             self._keep = (heat_p, paf_p)
         _lib.check(rc)
         self._n, self._hw = n, (h, w)
@@ -269,18 +288,31 @@ class PostProcessor:
 class PinnedBatch:
     """One pinned host block holding a batch's heat tensor directly followed by its PAF tensor (NCHW or NHWC):
     ``PostProcessor.run(b.heat, b.paf, ...)`` then moves both with a single host-to-device copy.
-    ``heat`` / ``paf`` are NumPy views to fill in place."""
+    ``heat`` / ``paf`` are views to fill in place: NumPy arrays for ``dtype`` 'float32' and 'float16', torch.bfloat16
+    CPU tensors for 'bfloat16' (NumPy has no bfloat16).  The 16-bit blocks are half the size and are widened to float32
+    on the device."""
 
-    def __init__(self, n: int, h: int, w: int, layout: str = "nchw", write_combined: bool = False):
+    _ITEMSIZE = {"float32": 4, "float16": 2, "bfloat16": 2}
+
+    def __init__(self, n: int, h: int, w: int, layout: str = "nchw", write_combined: bool = False, dtype: str = "float32"):
+        if dtype not in self._ITEMSIZE:
+            raise ValueError("dtype must be 'float32', 'float16' or 'bfloat16'")
+        if dtype == "bfloat16" and torch is None:
+            raise ValueError("a bfloat16 PinnedBatch needs torch (NumPy has no bfloat16)")
         self._ptr = C.c_void_p()
         nh, npf = n * h * w * _lib.HEAT_CH, n * h * w * _lib.PAF_CH
-        _lib.check(_lib.lib.ekp_host_alloc(C.byref(self._ptr), 4 * (nh + npf), int(bool(write_combined))))
-        buf = (C.c_float * (nh + npf)).from_address(self._ptr.value)
-        flat = np.frombuffer(buf, dtype=np.float32)
+        item = self._ITEMSIZE[dtype]
+        _lib.check(_lib.lib.ekp_host_alloc(C.byref(self._ptr), item * (nh + npf), int(bool(write_combined))))
+        buf = (C.c_uint8 * (item * (nh + npf))).from_address(self._ptr.value)
+        if dtype == "bfloat16":
+            flat = torch.frombuffer(buf, dtype=torch.bfloat16)
+        else:
+            flat = np.frombuffer(buf, dtype=np.float32 if dtype == "float32" else np.float16)
         shp = (lambda c: (n, c, h, w)) if layout == "nchw" else (lambda c: (n, h, w, c))
         self.heat = flat[:nh].reshape(shp(_lib.HEAT_CH))
         self.paf = flat[nh:].reshape(shp(_lib.PAF_CH))
-        self.nbytes = 4 * (nh + npf)
+        self.dtype = dtype
+        self.nbytes = item * (nh + npf)
 
     def close(self):
         if getattr(self, "_ptr", None) and self._ptr.value:
