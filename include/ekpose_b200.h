@@ -165,6 +165,31 @@ int ekp_results(ekp_ctx *ctx, int *num_humans, float *subset, int *n_peaks, ekp_
  * float32 [n, max_humans] = subset[18] / subset[19] (get_score, pafprocess.cpp:204-206). */
 int ekp_results_humans(ekp_ctx *ctx, int *num_humans, ekp_peak *parts, float *scores, unsigned *overflow);
 
+/* ---- drawing (SURVEY.md 8f row f2) --------------------------------------------------------------
+ * Paints the people of the last run onto n DEVICE frames uint8 [n, H, W, 3] (contiguous, in place), as the reference's
+ * draw_humans (lib/utils/common.py:252-275) paints each image's list[Human]: byte for byte.  Per human of the table, in
+ * table order, its part markers (cv2.circle radius 3, thickness 3) in part order, then its limbs (cv2.line thickness 3)
+ * in CocoPairsRender order; a pixel takes the colour of the last of them that covers it, CocoColors written to channels
+ * 0, 1, 2 in tuple order.  Coordinates are normalised by the last run's full-resolution map (8h x 8w; H x W of
+ * ekp_process_paf_dev's paf_mat), so frames of any size up to EKP_DRAW_MAX_SIDE a side work.  Pixels no marker or limb
+ * covers are not touched.  Asynchronous on `stream`, ordered after the run; no host wait.  Draws what the human table
+ * holds, overflow or not (ekp_results* report overflow).  Two kernel launches (counted in ekp_kernel_launches); a
+ * context-owned key buffer of n x H x W uint32 is allocated on first use and grown on demand.  The draw is ordered
+ * before the context's next run on any stream, so a run cannot overwrite the results the draw reads.
+ * EKP_ERR_STATE before any run; EKP_ERR_ARG for a NULL context or frames, n != ekp_last_batch(ctx), or H, W outside
+ * [1, EKP_DRAW_MAX_SIDE]. */
+#define EKP_DRAW_MAX_SIDE 16384
+int ekp_draw_humans(ekp_ctx *ctx, unsigned char *frames, int n, int H, int W, void *stream);
+
+/* Test hooks for the rasteriser of ekp_draw_humans: the same code, run serially on the CPU on HOST buffers (they are not a
+ * CPU path of ekp_draw_humans).  ekp_debug_raster_host sets mask[y][x] = 1 (uint8 [H, W]) for every pixel one primitive
+ * paints: kind 1 the part marker centred at (x0, y0), kind 2 the limb (x0, y0) - (x1, y1).  ekp_debug_draw_host paints
+ * the people of a human table (num_humans [n], parts ekp_peak [n, max_humans, 18] as ekp_results_humans writes it)
+ * normalised by a map_h x map_w map onto frames uint8 [n, H, W, 3], in drawing order. */
+int ekp_debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char *mask);
+int ekp_debug_draw_host(const int *num_humans, const ekp_peak *parts, int max_humans, int map_h, int map_w,
+                        unsigned char *frames, int n, int H, int W);
+
 /* The 13 distinct weights w[-12] .. w[0] of scipy.ndimage's Gaussian kernel for sigma = 3 as the context uploads them for
  * EKP_FRONTEND_REFERENCE_GAUSS (host-only; tests compare them with scipy's own array). */
 int ekp_scipy_gauss3_weights(double *out13);

@@ -21,6 +21,7 @@ OK, ERR_ARG, ERR_CUDA, ERR_CAPACITY, ERR_STATE = 0, -1, -2, -3, -4
 OVF_PEAKS, OVF_PART, OVF_CANDIDATES, OVF_HUMANS, OVF_BADPEAK = 1, 2, 4, 8, 16
 MAX_PART, MAX_CAND = 256, 2048                                              # EKP_MAX_PART / EKP_MAX_CAND (defaults)
 LIMIT_PEAKS, LIMIT_HUMANS, LIMIT_PART, LIMIT_CAND = 16384, 1024, 1024, 8192  # EKP_LIMIT_*
+DRAW_MAX_SIDE = 16384                                                       # EKP_DRAW_MAX_SIDE
 
 
 class EkpError(RuntimeError):
@@ -70,6 +71,9 @@ SIGNATURES = {
     "ekp_graph_launches": (C.c_longlong, [_vp]),
     "ekp_host_alloc": (_i, [C.POINTER(_vp), C.c_size_t, _i]),
     "ekp_host_free": (_i, [_vp]),
+    "ekp_draw_humans": (_i, [_vp, _vp, _i, _i, _i, _vp]),
+    "ekp_debug_raster_host": (_i, [_i, _i, _i, _i, _i, _i, _i, _vp]),
+    "ekp_debug_draw_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _i, _i]),
     # the reference operator surface, lib/pafprocess/pafprocess.h:53-59
     "process_paf": (_i, [_i, _i, _i, _vp, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "get_num_humans": (_i, []),

@@ -3,8 +3,8 @@
 Mirrors the output contract of /root/reference/lib/utils/common.py: ``Human`` (:51-63) with
 ``body_parts`` {part_idx: BodyPart} and ``score``; ``BodyPart`` (:277-298) with ``uidx``,
 ``part_idx``, normalised ``x``, ``y`` in [0, 1) and ``score``; the part enumeration (:6-25) and
-limb table (:27-30).  Drawing and the face / upper-body box heuristics of that file are host-side
-visualisation and out of scope (SURVEY.md section 8).
+limb table (:27-30).  Drawing (:252-275) is ``PostProcessor.draw_humans`` on the device (``ekp_draw_humans``); the
+face / upper-body box heuristics of that file are host-side visualisation and out of scope (SURVEY.md section 8).
 """
 from enum import Enum
 

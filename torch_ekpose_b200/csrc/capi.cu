@@ -51,6 +51,11 @@ cudaError_t launch_preprocess(const unsigned char* src, float* out, const int* x
                               cudaStream_t stream);
 cudaError_t launch_widen(const void* heat16, const void* paf16, size_t n_heat, size_t n_paf, int dtype, float* heat, float* paf,
                          cudaStream_t stream);
+cudaError_t launch_draw(const unsigned char* records, const ResultLayout& lay, int max_humans, int map_h, int map_w,
+                        unsigned char* frames, int n, int H, int W, unsigned* keys, unsigned epoch, cudaStream_t stream);
+void debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask);
+void debug_draw_host(const int* num_humans, const ekp_peak* parts, int max_humans, int map_h, int map_w,
+                     unsigned char* frames, int n, int H, int W);
 }  // namespace ekp
 
 using namespace ekp;
@@ -189,6 +194,11 @@ struct ekp_ctx {
     Conn* conns = nullptr;          // [max_batch][19][max_part]
     int* n_conns = nullptr;         // [max_batch][19]
     unsigned char* records = nullptr;  // [max_batch] packed result records (ResultLayout)
+    const unsigned char* last_records = nullptr;  // where the last run's assembly wrote them (records, or pinned host)
+    int map_h = 0, map_w = 0;       // the last run's full-resolution map, by which ekp_draw_humans normalises
+    unsigned* draw_keys = nullptr;  // ekp_draw_humans' per-pixel keys (lazily, grown on demand)
+    size_t draw_keys_cap = 0;       // pixels
+    unsigned draw_epoch = 0;        // draws since the keys were last cleared (the high 16 bits of every key)
     ResultLayout lay = {};
     float* in_block = nullptr;      // staging for the host-buffer entry point: [heat | paf] of one batch, contiguous
                                     // (also where 16-bit inputs are widened to)
@@ -234,7 +244,8 @@ static int ctx_free(ekp_ctx* c) {
     if (!c) return EKP_OK;
     cudaSetDevice(c->device);
     void* dev[] = {c->raw, c->raw_count, c->line, c->part_off, c->n_peaks, c->conns, c->n_conns, c->records,
-                   c->in_block, c->in_block16, c->mat_heat, c->mat_paf, c->ax, c->ay, c->cubic, c->gauss, c->prep_tab};
+                   c->in_block, c->in_block16, c->mat_heat, c->mat_paf, c->ax, c->ay, c->cubic, c->gauss, c->prep_tab,
+                   c->draw_keys};
     for (void* p : dev) if (p) cudaFree(p);
     void* host[] = {c->h_records, c->h_line};
     for (void* p : host) if (p) cudaFreeHost(p);
@@ -402,6 +413,7 @@ static int run_connect_assemble(ekp_ctx* c, int n, const PafSource& paf, int h1,
     ap.line = c->line; ap.max_peaks = c->max_peaks; ap.n_peaks = c->n_peaks; ap.part_off = c->part_off; ap.conns = c->conns;
     ap.n_conns = c->n_conns; ap.max_part = c->max_part; ap.max_humans = c->max_humans; ap.conn_cap = 0; ap.overflow = c->overflow;
     ap.records = records_direct ? records_direct : c->records; ap.lay = c->lay;
+    c->last_records = ap.records;
     ConnectParams cp;
     cp.line = c->line; cp.part_off = c->part_off; cp.max_peaks = c->max_peaks; cp.max_part = c->max_part; cp.max_cand = c->max_cand;
     cp.paf = paf; cp.h1 = h1; cp.conns = c->conns; cp.n_conns = c->n_conns; cp.overflow = c->overflow;
@@ -542,6 +554,7 @@ static int submit_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
         c->launches += hit->kernels;
         c->graph_launches += 1;
     }
+    c->map_h = 8 * a.h; c->map_w = 8 * a.w;
     return finish_submit(c, a.n, st);
 }
 
@@ -688,6 +701,7 @@ extern "C" int ekp_process_paf_dev(ekp_ctx* c, const float* peaks, const int* n_
     src.pair_base = nullptr; src.ids_are_rows = 0;
     int rc = run_back_half(c, n, /*id_from_key=*/1, src, h1, st);
     if (rc) return rc;
+    c->map_h = H; c->map_w = W;
     return finish_submit(c, n, st);
 }
 
@@ -747,6 +761,55 @@ extern "C" int ekp_results_humans(ekp_ctx* c, int* num_humans, ekp_peak* parts, 
         if (scores) memcpy(scores + (size_t) i * mh, rec + c->lay.off_hscore, sizeof(float) * (size_t) hd->num_humans);
     }
     return overflow_status(c);
+}
+
+// ---- drawing (draw.cu) --------------------------------------------------------------------------
+extern "C" int ekp_draw_humans(ekp_ctx* c, unsigned char* frames, int n, int H, int W, void* stream) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_draw_humans: NULL context");
+    if (!c->has_run) return fail(EKP_ERR_STATE, "ekp_draw_humans: no run has been submitted on this context");
+    if (!frames) return fail(EKP_ERR_ARG, "ekp_draw_humans: NULL frames");
+    if (n != c->last_n) return fail(EKP_ERR_ARG, "ekp_draw_humans: %d frames for a run of %d images", n, c->last_n);
+    if (H < 1 || W < 1 || H > EKP_DRAW_MAX_SIDE || W > EKP_DRAW_MAX_SIDE)
+        return fail(EKP_ERR_ARG, "ekp_draw_humans: frame %dx%d outside [1x1, %dx%d]", H, W, EKP_DRAW_MAX_SIDE, EKP_DRAW_MAX_SIDE);
+    cudaStream_t st = (cudaStream_t) stream;
+    CU(cudaSetDevice(c->device));
+    if (c->last_stream != st) CU(cudaStreamWaitEvent(st, c->done, 0));  // the records of the run, the keys of earlier draws
+    const size_t pixels = (size_t) n * H * W;
+    if (c->draw_keys_cap < pixels) {
+        CU(cudaEventSynchronize(c->done));  // no draw in flight may still use the old keys
+        if (c->draw_keys) { cudaFree(c->draw_keys); c->draw_keys = nullptr; }
+        c->draw_keys_cap = 0;
+        CU(cudaMalloc((void**) &c->draw_keys, sizeof(unsigned) * pixels));
+        c->draw_keys_cap = pixels;
+        c->draw_epoch = 0xffff;  // cleared below
+    }
+    if (c->draw_epoch == 0xffff) {  // the epoch would wrap: keys of old draws could equal or exceed this draw's
+        CU(cudaMemsetAsync(c->draw_keys, 0, sizeof(unsigned) * c->draw_keys_cap, st));
+        c->draw_epoch = 0;
+    }
+    c->draw_epoch += 1;
+    CU(launch_draw(c->last_records, c->lay, c->max_humans, c->map_h, c->map_w, frames, n, H, W, c->draw_keys, c->draw_epoch, st));
+    c->launches += 2;
+    // a later run on any stream waits for this draw before it overwrites the records (submit_batch)
+    CU(cudaEventRecord(c->done, st));
+    c->last_stream = st;
+    return EKP_OK;
+}
+
+extern "C" int ekp_debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask) {
+    if (!mask || (kind != 1 && kind != 2) || H < 1 || W < 1 || H > EKP_DRAW_MAX_SIDE || W > EKP_DRAW_MAX_SIDE)
+        return fail(EKP_ERR_ARG, "ekp_debug_raster_host: bad arguments");
+    debug_raster_host(kind, x0, y0, x1, y1, H, W, mask);
+    return EKP_OK;
+}
+
+extern "C" int ekp_debug_draw_host(const int* num_humans, const ekp_peak* parts, int max_humans, int map_h, int map_w,
+                                   unsigned char* frames, int n, int H, int W) {
+    if (!num_humans || !parts || !frames || n < 1 || max_humans < 1 || max_humans > EKP_LIMIT_HUMANS || map_h < 1 || map_w < 1 ||
+        H < 1 || W < 1 || H > EKP_DRAW_MAX_SIDE || W > EKP_DRAW_MAX_SIDE)
+        return fail(EKP_ERR_ARG, "ekp_debug_draw_host: bad arguments");
+    debug_draw_host(num_humans, parts, max_humans, map_h, map_w, frames, n, H, W);
+    return EKP_OK;
 }
 
 extern "C" int ekp_debug_std_sort(ekp_ctx* c, float* scores_dev, unsigned* tags_dev, int n, void* stream) {

@@ -10,9 +10,10 @@ whole batch of equally sized frames: the raw uint8 frames are uploaded once, ``p
 normalisation are ONE CUDA kernel (``ekp_preprocess``, bit-identical to cv2's 8-bit fixed-point
 resize and the reference's float32 normalisation), the model runs one forward pass, and its outputs
 stay on the device in the layout it emits (NCHW): no device-to-host copy, no transpose.
-``infer_humans`` feeds them straight to the CUDA post-processing on the same device.  There is no
-host implementation of any of this in the package; the model itself is the caller's (cuDNN through
-PyTorch; out of scope).
+``infer_humans`` feeds them straight to the CUDA post-processing on the same device, and
+``infer_and_draw`` also paints the people onto the uploaded frames (``ekp_draw_humans``, byte for
+byte the reference's ``draw_humans``).  There is no host implementation of any of this in the
+package; the model itself is the caller's (cuDNN through PyTorch; out of scope).
 """
 from __future__ import annotations
 
@@ -35,37 +36,42 @@ def _device_index(device) -> int:
     return dev.index if dev.index is not None else torch.cuda.current_device()
 
 
-def get_outputs_batched(images, model, preprocess: str, device):
-    """Batched ``get_outputs``: returns (pafs [n,38,h,w], heatmaps [n,19,h,w], im_scale) with the two
-    tensors left on ``device``.  ``images``: a sequence of equally sized uint8 BGR frames [H,W,3]
-    (frames of one stream) or one CUDA uint8 tensor [n,H,W,3] already on ``device``."""
+def _upload(images, idx: int):
+    """The frames as a CUDA uint8 tensor [n,H,W,3] on cuda:``idx``: a CUDA tensor already there as it is, anything
+    else copied there once."""
     import torch
-    idx = _device_index(device)
     dev = torch.device("cuda", idx)
     if isinstance(images, torch.Tensor):
         frames = images
         if not frames.is_cuda or frames.device.index != idx:
             frames = frames.to(dev, non_blocking=True)
-    else:
-        if len({im.shape for im in images}) != 1:
-            raise ValueError("get_outputs_batched needs equally sized images (batch them per resolution)")
-        frames = torch.from_numpy(np.stack(images)).to(dev, non_blocking=True)
+        return frames
+    if len({im.shape for im in images}) != 1:
+        raise ValueError("get_outputs_batched needs equally sized images (batch them per resolution)")
+    return torch.from_numpy(np.stack(images)).to(dev, non_blocking=True)
+
+
+def _forward(frames, model, preprocess: str, idx: int):
+    import torch
     pp = _prep_ctx.get(idx)
     if pp is None:
         pp = _prep_ctx[idx] = PostProcessor(device=idx, max_batch=1, max_h=5, max_w=5, max_peaks=16, max_humans=4)
-    with torch.cuda.device(dev):
+    with torch.cuda.device(idx):
         batch_var, scale = pp.preprocess(frames, mode=preprocess)
         with torch.no_grad():
             predicted, _ = model(batch_var)
     return predicted[-2], predicted[-1], scale
 
 
-def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, frontend: str = "reference",
-                 thr: float = 0.15) -> List[list]:
-    """images -> per-image list[Human]: GPU preprocessing, one forward pass, post-processing on the same GPU
-    (the network's outputs never leave the device, and 16-bit outputs of a model under torch.autocast are taken as
-    they are).  ``frontend='reference'`` gives the reference's people."""
-    pafs, heats, _ = get_outputs_batched(images, model, preprocess, device)
+def get_outputs_batched(images, model, preprocess: str, device):
+    """Batched ``get_outputs``: returns (pafs [n,38,h,w], heatmaps [n,19,h,w], im_scale) with the two
+    tensors left on ``device``.  ``images``: a sequence of equally sized uint8 BGR frames [H,W,3]
+    (frames of one stream) or one CUDA uint8 tensor [n,H,W,3] already on ``device``."""
+    idx = _device_index(device)
+    return _forward(_upload(images, idx), model, preprocess, idx)
+
+
+def _postprocess(heats, pafs, frontend: str, thr: float) -> PostProcessor:
     n, _, h, w = heats.shape
     idx = heats.device.index
     key = (idx, n, h, w)
@@ -74,9 +80,29 @@ def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, f
         pp = _pp_cache[key] = PostProcessor(device=idx, max_batch=n, max_h=h, max_w=w, max_peaks=2048, max_humans=128)
     _last_pp[0] = pp
     pp.run(heats, pafs, layout="nchw", frontend=frontend, thr=thr)   # bf16 / fp16 under autocast: widened on the device
-    return pp.humans()
+    return pp
+
+
+def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, frontend: str = "reference",
+                 thr: float = 0.15) -> List[list]:
+    """images -> per-image list[Human]: GPU preprocessing, one forward pass, post-processing on the same GPU
+    (the network's outputs never leave the device, and 16-bit outputs of a model under torch.autocast are taken as
+    they are).  ``frontend='reference'`` gives the reference's people."""
+    pafs, heats, _ = get_outputs_batched(images, model, preprocess, device)
+    return _postprocess(heats, pafs, frontend, thr).humans()
+
+
+def infer_and_draw(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15):
+    """``infer_humans`` followed by the reference's ``draw_humans`` on every frame, all on the GPU: returns the drawn
+    frames, a CUDA uint8 tensor [n,H,W,3] on ``device``.  Host frames are drawn on the copy uploaded for the
+    preprocessing; a CUDA tensor on ``device`` (contiguous) is drawn in place.  The people stay available through
+    ``last_postprocessor()``; the call does not wait for the device."""
+    idx = _device_index(device)
+    frames = _upload(images, idx)
+    pafs, heats, _ = _forward(frames, model, preprocess, idx)
+    return _postprocess(heats, pafs, frontend, thr).draw_humans(frames)
 
 
 def last_postprocessor():
-    """The context the last ``infer_humans`` call used (stage timing in the benchmark)."""
+    """The context the last ``infer_humans`` / ``infer_and_draw`` call used (stage timing in the benchmark)."""
     return _last_pp[0]

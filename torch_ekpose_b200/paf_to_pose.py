@@ -238,6 +238,26 @@ class PostProcessor:
             out.append(humans)
         return out
 
+    def draw_humans(self, frames, stream=None):
+        """Paints the people of the last run onto ``frames``, a contiguous CUDA uint8 tensor [n, H, W, 3] on this
+        context's device with one frame per image of the run, in place, and returns it: byte for byte what the
+        reference's ``draw_humans(frame, humans)`` (lib/utils/common.py:252-275, imgcopy=False) paints with the
+        people ``humans()`` returns.  Frames of any size work (coordinates are normalised by the run's map, as in
+        the reference).  Asynchronous on ``stream`` (default: the current stream), ordered after the run."""
+        if not (_is_tensor(frames) and frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 4 and
+                frames.shape[3] == 3 and frames.is_contiguous()):
+            raise ValueError("frames must be a contiguous CUDA uint8 tensor [n, H, W, 3]")
+        if frames.device.index != self.device:
+            raise ValueError(f"frames are on cuda:{frames.device.index}, context on cuda:{self.device}")
+        n, H, W, _ = frames.shape
+        rows = self._rows()
+        if rows and n != rows:
+            raise ValueError(f"{n} frames for a run of {rows} images")
+        if not (1 <= H <= _lib.DRAW_MAX_SIDE and 1 <= W <= _lib.DRAW_MAX_SIDE):
+            raise ValueError(f"frames of {H}x{W} outside [1x1, {_lib.DRAW_MAX_SIDE}x{_lib.DRAW_MAX_SIDE}]")
+        _lib.check(_lib.lib.ekp_draw_humans(self._ctx, frames.data_ptr(), n, H, W, self._stream(stream)))
+        return frames
+
     def set_timing(self, enable: bool) -> None:
         _lib.check(_lib.lib.ekp_set_timing(self._ctx, int(bool(enable))))
 
