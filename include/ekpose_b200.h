@@ -17,7 +17,9 @@
  * 2. A handle-based batched API on DEVICE (or pinned host) tensors that also covers the
  *    Python-side preprocessing of the reference (lib/utils/paf_to_pose.py: find_peaks :26-36,
  *    NMS :60-133, the upsampling of paf_to_pose_cpp :356-359) as CUDA stages 1-3, so a whole
- *    batch goes from the network's stride-8 outputs to people in one call.
+ *    batch goes from the network's stride-8 outputs to people in one call.  The people come back as host tables
+ *    (ekp_results, ekp_results_humans: these wait for the run) or into caller-owned device buffers, ordered on a
+ *    stream with no host wait (ekp_results_device).
  *
  * All functions return EKP_OK (0) or a negative ekp_status; ekp_last_error() returns a
  * thread-local human-readable message for the last failure.  Nothing aborts.
@@ -164,6 +166,29 @@ int ekp_results(ekp_ctx *ctx, int *num_humans, float *subset, int *n_peaks, ekp_
  * i.e. get_part_cid / get_part_x / get_part_y / get_part_score in one table, and the human score
  * float32 [n, max_humans] = subset[18] / subset[19] (get_score, pafprocess.cpp:204-206). */
 int ekp_results_humans(ekp_ctx *ctx, int *num_humans, ekp_peak *parts, float *scores, unsigned *overflow);
+
+/* ---- results on the device ---------------------------------------------------------------------
+ * The tables of ekp_results / ekp_results_humans written into caller-owned DEVICE buffers instead of host arrays, so a
+ * caller that keeps the people on the GPU (a tracker, a second model, crops) neither waits for the run nor copies them
+ * back.  Every pointer is a device pointer, 4-byte aligned, and may be NULL (that table is not written). */
+typedef struct ekp_device_results {
+    int *num_humans;      /* [n]                     people per image */
+    unsigned *overflow;   /* [n]                     EKP_OVF_* bits */
+    int *n_peaks;         /* [n]                     peaks per image */
+    float *subset;        /* [n, max_humans, 20]     as ekp_results */
+    ekp_peak *parts;      /* [n, max_humans, 18]     as ekp_results_humans */
+    float *scores;        /* [n, max_humans]         as ekp_results_humans */
+} ekp_device_results;
+/* Writes the last run's tables into `out` for its n = ekp_last_batch(ctx) images.  Rows from num_humans[i] up to
+ * max_humans are written as zero bytes, so each table copied to the host equals the host call's byte for byte, padding
+ * included.  One kernel launch (counted in ekp_kernel_launches; not part of the batch's CUDA graph), asynchronous on
+ * `stream` and ordered like ekp_draw_humans: after the run (an export on another stream waits for it), and before the
+ * context's next run on any stream.  It never waits on the host and never allocates.  Works after every batched entry
+ * point (ekp_postprocess*, ekp_postprocess_host*, ekp_process_paf_dev).
+ * Overflow does not fail the call (nothing is known about it at call time): the bits land in `overflow`, and the caller
+ * checks them.  EKP_ERR_STATE before any run; EKP_ERR_ARG for a NULL context or out, n != ekp_last_batch(ctx) or a
+ * pointer that is not 4-byte aligned.  All pointers NULL: EKP_OK, nothing is launched. */
+int ekp_results_device(ekp_ctx *ctx, int n, const ekp_device_results *out, void *stream);
 
 /* ---- drawing (SURVEY.md 8f row f2) --------------------------------------------------------------
  * Paints the people of the last run onto n DEVICE frames uint8 [n, H, W, 3] (contiguous, in place), as the reference's

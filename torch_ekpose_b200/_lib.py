@@ -38,6 +38,11 @@ class Peak(C.Structure):  # ekp_peak
     _fields_ = [("x", C.c_int), ("y", C.c_int), ("score", C.c_float), ("id", C.c_int)]
 
 
+class DeviceResults(C.Structure):  # ekp_device_results: device pointers, None = that table is not written
+    _fields_ = [("num_humans", C.c_void_p), ("overflow", C.c_void_p), ("n_peaks", C.c_void_p), ("subset", C.c_void_p),
+                ("parts", C.c_void_p), ("scores", C.c_void_p)]
+
+
 # every symbol include/ekpose_b200.h declares: (restype, argtypes)
 _vp, _i, _f = C.c_void_p, C.c_int, C.c_float
 SIGNATURES = {
@@ -53,6 +58,7 @@ SIGNATURES = {
     "ekp_process_paf_dev": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "ekp_results": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "ekp_results_humans": (_i, [_vp, _vp, _vp, _vp, _vp]),
+    "ekp_results_device": (_i, [_vp, _i, C.POINTER(DeviceResults), _vp]),
     "ekp_scipy_gauss3_weights": (_i, [_vp]),
     "ekp_debug_std_sort": (_i, [_vp, _vp, _vp, _i, _vp]),
     "ekp_results_parts": (_i, [_vp, _vp]),

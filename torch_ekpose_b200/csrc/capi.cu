@@ -635,7 +635,20 @@ extern "C" int ekp_results_humans(ekp_ctx* c, int* num_humans, ekp_peak* parts, 
     return overflow_status(c);
 }
 
-// ---- drawing (draw.cu) --------------------------------------------------------------------------
+// ---- readers of the last run's records on the device (draw.cu, results_device.cu) ----------------------------------
+// Puts what enqueue() issues on `st` after the last run (and after earlier readers: the draw's keys), and the context's
+// next run on any stream after it, so that run cannot overwrite the records while they are read (submit_batch waits for
+// `done`).  No host wait.
+static int after_run(ekp_ctx* c, cudaStream_t st, const std::function<int()>& enqueue) {
+    CU(cudaSetDevice(c->device));
+    if (c->last_stream != st) CU(cudaStreamWaitEvent(st, c->done, 0));
+    int rc = enqueue();
+    if (rc) return rc;
+    CU(cudaEventRecord(c->done, st));
+    c->last_stream = st;
+    return EKP_OK;
+}
+
 extern "C" int ekp_draw_humans(ekp_ctx* c, unsigned char* frames, int n, int H, int W, void* stream) {
     if (!c) return fail(EKP_ERR_ARG, "ekp_draw_humans: NULL context");
     if (!c->has_run) return fail(EKP_ERR_STATE, "ekp_draw_humans: no run has been submitted on this context");
@@ -644,26 +657,42 @@ extern "C" int ekp_draw_humans(ekp_ctx* c, unsigned char* frames, int n, int H, 
     if (H < 1 || W < 1 || H > EKP_DRAW_MAX_SIDE || W > EKP_DRAW_MAX_SIDE)
         return fail(EKP_ERR_ARG, "ekp_draw_humans: frame %dx%d outside [1x1, %dx%d]", H, W, EKP_DRAW_MAX_SIDE, EKP_DRAW_MAX_SIDE);
     cudaStream_t st = (cudaStream_t) stream;
-    CU(cudaSetDevice(c->device));
-    if (c->last_stream != st) CU(cudaStreamWaitEvent(st, c->done, 0));  // the records of the run, the keys of earlier draws
-    const size_t pixels = (size_t) n * H * W;
-    if (c->draw_keys_cap < pixels) {
-        CU(cudaEventSynchronize(c->done));  // no draw in flight may still use the old keys
-        int rc = grow(c->draw_keys, c->draw_keys_cap, pixels);
-        if (rc) return rc;
-        c->draw_epoch = 0xffff;  // cleared below
+    return after_run(c, st, [&]() {
+        const size_t pixels = (size_t) n * H * W;
+        if (c->draw_keys_cap < pixels) {
+            CU(cudaEventSynchronize(c->done));  // no draw in flight may still use the old keys
+            int rc = grow(c->draw_keys, c->draw_keys_cap, pixels);
+            if (rc) return rc;
+            c->draw_epoch = 0xffff;  // cleared below
+        }
+        if (c->draw_epoch == 0xffff) {  // the epoch would wrap: keys of old draws could equal or exceed this draw's
+            CU(cudaMemsetAsync(c->draw_keys, 0, sizeof(unsigned) * c->draw_keys_cap, st));
+            c->draw_epoch = 0;
+        }
+        c->draw_epoch += 1;
+        CU(launch_draw(c->last_records, c->lay, c->max_humans, c->map_h, c->map_w, frames, n, H, W, c->draw_keys, c->draw_epoch, st));
+        c->launches += 2;
+        return (int) EKP_OK;
+    });
+}
+
+extern "C" int ekp_results_device(ekp_ctx* c, int n, const ekp_device_results* out, void* stream) {
+    if (!c || !out) return fail(EKP_ERR_ARG, "ekp_results_device: NULL %s", c ? "out" : "context");
+    if (!c->has_run) return fail(EKP_ERR_STATE, "ekp_results_device: no run has been submitted on this context");
+    if (n != c->last_n) return fail(EKP_ERR_ARG, "ekp_results_device: tables for %d images, the run had %d", n, c->last_n);
+    const void* ptrs[] = {out->num_humans, out->overflow, out->n_peaks, out->subset, out->parts, out->scores};
+    bool any = false;
+    for (const void* p : ptrs) {
+        if (reinterpret_cast<uintptr_t>(p) & 3u) return fail(EKP_ERR_ARG, "ekp_results_device: a pointer is not 4-byte aligned");
+        any = any || p;
     }
-    if (c->draw_epoch == 0xffff) {  // the epoch would wrap: keys of old draws could equal or exceed this draw's
-        CU(cudaMemsetAsync(c->draw_keys, 0, sizeof(unsigned) * c->draw_keys_cap, st));
-        c->draw_epoch = 0;
-    }
-    c->draw_epoch += 1;
-    CU(launch_draw(c->last_records, c->lay, c->max_humans, c->map_h, c->map_w, frames, n, H, W, c->draw_keys, c->draw_epoch, st));
-    c->launches += 2;
-    // a later run on any stream waits for this draw before it overwrites the records (submit_batch)
-    CU(cudaEventRecord(c->done, st));
-    c->last_stream = st;
-    return EKP_OK;
+    if (!any) return EKP_OK;
+    cudaStream_t st = (cudaStream_t) stream;
+    return after_run(c, st, [&]() {
+        CU(launch_results_export(c->last_records, c->lay, c->max_humans, n, *out, st));
+        c->launches += 1;
+        return (int) EKP_OK;
+    });
 }
 
 extern "C" int ekp_debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask) {

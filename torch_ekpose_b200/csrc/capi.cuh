@@ -42,6 +42,8 @@ cudaError_t launch_widen(const void* heat16, const void* paf16, size_t n_heat, s
                          cudaStream_t stream);
 cudaError_t launch_draw(const unsigned char* records, const ResultLayout& lay, int max_humans, int map_h, int map_w,
                         unsigned char* frames, int n, int H, int W, unsigned* keys, unsigned epoch, cudaStream_t stream);
+cudaError_t launch_results_export(const unsigned char* records, const ResultLayout& lay, int max_humans, int n,
+                                  const ekp_device_results& out, cudaStream_t stream);
 void debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask);
 void debug_draw_host(const int* num_humans, const ekp_peak* parts, int max_humans, int map_h, int map_w,
                      unsigned char* frames, int n, int H, int W);

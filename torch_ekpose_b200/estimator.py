@@ -12,7 +12,8 @@ resize and the reference's float32 normalisation), the model runs one forward pa
 stay on the device in the layout it emits (NCHW): no device-to-host copy, no transpose.
 ``infer_humans`` feeds them straight to the CUDA post-processing on the same device, and
 ``infer_and_draw`` also paints the people onto the uploaded frames (``ekp_draw_humans``, byte for
-byte the reference's ``draw_humans``).  There is no host implementation of any of this in the
+byte the reference's ``draw_humans``), and ``infer_human_tensors`` returns the people as CUDA tensors
+(``ekp_results_device``) without waiting for the device.  There is no host implementation of any of this in the
 package; the model itself is the caller's (cuDNN through PyTorch; out of scope).
 """
 from __future__ import annotations
@@ -92,6 +93,16 @@ def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, f
     return _postprocess(heats, pafs, frontend, thr).humans()
 
 
+def infer_human_tensors(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15,
+                        subset: bool = False):
+    """``infer_humans`` with the people left on the GPU: returns (tensors, im_scale), ``tensors`` being the dict of
+    CUDA tensors ``PostProcessor.result_tensors(subset=subset)`` returns (per image num_humans, overflow, n_peaks,
+    the part table, part and human scores) and ``im_scale`` that of ``get_outputs_batched``.  Nothing waits for the
+    device and nothing raises on a capacity overflow: the caller checks ``tensors['overflow']``."""
+    pafs, heats, im_scale = get_outputs_batched(images, model, preprocess, device)
+    return _postprocess(heats, pafs, frontend, thr).result_tensors(subset=subset), im_scale
+
+
 def infer_and_draw(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15):
     """``infer_humans`` followed by the reference's ``draw_humans`` on every frame, all on the GPU: returns the drawn
     frames, a CUDA uint8 tensor [n,H,W,3] on ``device``.  Host frames are drawn on the copy uploaded for the
@@ -104,5 +115,5 @@ def infer_and_draw(images, model, preprocess: str, device, frontend: str = "refe
 
 
 def last_postprocessor():
-    """The context the last ``infer_humans`` / ``infer_and_draw`` call used (stage timing in the benchmark)."""
+    """The context the last ``infer_humans`` / ``infer_and_draw`` / ``infer_human_tensors`` call used (stage timing in the benchmark)."""
     return _last_pp[0]

@@ -217,6 +217,56 @@ class PostProcessor:
         _lib.check(_lib.lib.ekp_results_humans(self._ctx, num.ctypes.data, parts.ctypes.data, scores.ctypes.data, None))
         return num, parts, scores
 
+    def _result_specs(self, n: int, subset: bool):
+        mh = self.max_humans
+        specs = [("num_humans", (n,), torch.int32), ("overflow", (n,), torch.int32), ("n_peaks", (n,), torch.int32),
+                 ("parts", (n, mh, _lib.NUM_PART, 4), torch.int32), ("scores", (n, mh), torch.float32)]
+        if subset:
+            specs.append(("subset", (n, mh, _lib.SUBSET_COLS), torch.float32))
+        return specs
+
+    def result_tensors(self, *, subset: bool = False, out: Optional[dict] = None, stream=None) -> dict:
+        """The tables of the last run as CUDA tensors on this context's device, without waiting for the device: the
+        export is one kernel on ``stream`` (default: the current stream), ordered after the run and before this
+        context's next run on any stream.
+
+        Returns a dict of ``num_humans`` int32 [n], ``overflow`` int32 [n] (EKP_OVF_* bits), ``n_peaks`` int32 [n],
+        ``parts`` int32 [n, max_humans, 18, 4] (x, y, score bits, id; id -1 = absent, as ``human_tables``),
+        ``part_score`` float32 [n, max_humans, 18] (the view ``parts[..., 2].view(torch.float32)``), ``scores``
+        float32 [n, max_humans] and, with ``subset=True``, ``subset`` float32 [n, max_humans, 20] (as ``results``).
+        Rows from ``num_humans[i]`` on are zero, so each tensor copied to the host equals the host table byte for byte.
+
+        This never raises on a capacity overflow (nothing is known about it when the call returns): the caller checks
+        ``overflow``, where a non-zero entry means that image's tables were cut.  New tensors are allocated under the
+        export's stream; ``out=`` takes the dict of an earlier call and writes into its tensors instead (ValueError if
+        their shape, dtype, device or contiguity does not fit this run), e.g. to keep a ring of buffers with no
+        allocation per batch."""
+        n = self._rows()
+        if not n:
+            raise _lib.EkpError(_lib.ERR_STATE, "result_tensors: no run has been submitted on this context")
+        dev = torch.device("cuda", self.device)
+        specs = self._result_specs(n, subset)
+        if out is None:
+            if stream is None:
+                st = torch.cuda.current_stream(dev)
+            elif isinstance(stream, torch.cuda.Stream):
+                st = stream
+            else:
+                st = torch.cuda.ExternalStream(int(getattr(stream, "cuda_stream", stream)), device=dev)
+            with torch.cuda.device(dev), torch.cuda.stream(st):
+                out = {name: torch.empty(shape, dtype=dt, device=dev) for name, shape, dt in specs}
+            stream = st
+        else:
+            for name, shape, dt in specs:
+                t = out.get(name) if isinstance(out, dict) else None
+                if not (_is_tensor(t) and t.device == dev and t.dtype == dt and tuple(t.shape) == shape and t.is_contiguous()):
+                    raise ValueError(f"out[{name!r}] must be a contiguous {dt} tensor {list(shape)} on {dev}")
+        tabs = _lib.DeviceResults(*(out[k].data_ptr() if k in out and (k != "subset" or subset) else None
+                                    for k in ("num_humans", "overflow", "n_peaks", "subset", "parts", "scores")))
+        _lib.check(_lib.lib.ekp_results_device(self._ctx, n, C.byref(tabs), self._stream(stream)))
+        out["part_score"] = out["parts"][..., 2].view(torch.float32)
+        return out
+
     def humans(self) -> List[List[Human]]:
         """Per image the list[Human] the reference builds at paf_to_pose.py:361-378."""
         num, parts, scores = self.human_tables()
