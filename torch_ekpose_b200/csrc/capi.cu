@@ -273,6 +273,18 @@ static int ensure_tables(ekp_ctx* c, int h, int w, cudaStream_t stream) {
     return EKP_OK;
 }
 
+// The plane kernels (dense_plane_kernel, ref_scan_kernel<true>) run for every map whose plane fits in 200 KB of shared
+// memory.  ekp_create sizes their limits for the context's largest map only, and leaves the 48 KB default when that plane
+// is over 200 KB, so a smaller map's launch would be refused.  Raises the limits to this shape's planes (the functions only
+// ever raise them), once per shape and outside any stream capture.
+static int ensure_plane_limits(ekp_ctx* c, int h, int w) {
+    if (c->plane_h == h && c->plane_w == w) return EKP_OK;
+    CU(configure_dense_plane(h, w));
+    CU(configure_ref_frontend(h, w));
+    c->plane_h = h; c->plane_w = w;
+    return EKP_OK;
+}
+
 static int check_shape(const ekp_ctx* c, int n, int h, int w, int layout, const char* who) {
     if (!c) return fail(EKP_ERR_ARG, "%s: NULL context", who);
     if (n < 1 || n > c->max_batch) return fail(EKP_ERR_ARG, "%s: batch %d outside [1, %d]", who, n, c->max_batch);
@@ -448,10 +460,12 @@ static int submit_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
         int rc = ensure_tables(c, a.h, a.w, st);
         if (rc) return rc;
     }
+    int rc = ensure_plane_limits(c, a.h, a.w);
+    if (rc) return rc;
     GraphKey key = {};
     key.batch = a;
     const unsigned long long epoch = a.heat_host ? g_host_frees.load(std::memory_order_acquire) : 0;
-    int rc = launch_cached(c, key, epoch, st, [&](cudaStream_t q) { return enqueue_batch(c, a, q); });
+    rc = launch_cached(c, key, epoch, st, [&](cudaStream_t q) { return enqueue_batch(c, a, q); });
     if (rc) return rc;
     c->map_h = 8 * a.h; c->map_w = 8 * a.w;
     return finish_submit(c, a.n, st);

@@ -102,6 +102,7 @@ struct ekp_ctx {
     float* ax = nullptr;            // dense taps for (tab_h, tab_w)
     float* ay = nullptr;
     int tab_h = 0, tab_w = 0;
+    int plane_h = 0, plane_w = 0;   // the map shape the plane kernels' shared-memory limits were last raised for
     float* cubic = nullptr;         // [8][4]
     double* gauss = nullptr;        // [13]
     char* prep_tab = nullptr;       // resize tables of the input side for (prep_sh, prep_sw, prep_dest)
