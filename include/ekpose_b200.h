@@ -19,7 +19,8 @@
  *    NMS :60-133, the upsampling of paf_to_pose_cpp :356-359) as CUDA stages 1-3, so a whole
  *    batch goes from the network's stride-8 outputs to people in one call.  The people come back as host tables
  *    (ekp_results, ekp_results_humans: these wait for the run) or into caller-owned device buffers, ordered on a
- *    stream with no host wait (ekp_results_device).
+ *    stream with no host wait (ekp_results_device, ekp_results_device_peaks).  A caller that reads them only on the
+ *    device can also skip each batch's copy of the result records to the host (ekp_set_host_copy).
  *
  * All functions return EKP_OK (0) or a negative ekp_status; ekp_last_error() returns a
  * thread-local human-readable message for the last failure.  Nothing aborts.
@@ -189,6 +190,29 @@ typedef struct ekp_device_results {
  * checks them.  EKP_ERR_STATE before any run; EKP_ERR_ARG for a NULL context or out, n != ekp_last_batch(ctx) or a
  * pointer that is not 4-byte aligned.  All pointers NULL: EKP_OK, nothing is launched. */
 int ekp_results_device(ekp_ctx *ctx, int n, const ekp_device_results *out, void *stream);
+
+/* The part-sorted peak table of the last run in caller-owned DEVICE buffers (4-byte aligned; NULL: not written):
+ * the device counterpart of ekp_results' n_peaks / peaks_line and ekp_results_parts. */
+typedef struct ekp_device_peaks {
+    int *n_peaks;         /* [n]                     peaks per image */
+    ekp_peak *peaks;      /* [n, max_peaks]          part-sorted peak table, as ekp_results' peaks_line */
+    int *part_off;        /* [n, 19]                 as ekp_results_parts */
+} ekp_device_peaks;
+/* Writes the last run's peak tables into `out`: one kernel launch, ordered and checked exactly like ekp_results_device
+ * (same error codes; all pointers NULL: EKP_OK, nothing is launched).  Rows from min(n_peaks[i], max_peaks) up to
+ * max_peaks are written as zero bytes, so the table copied to the host equals ekp_results' peaks_line padding
+ * included. */
+int ekp_results_device_peaks(ekp_ctx *ctx, int n, const ekp_device_peaks *out, void *stream);
+
+/* Whether batches end with the device-to-host copy of their result records.  enable != 0 (the default): every batch
+ * of ekp_postprocess*, ekp_postprocess_host* and ekp_process_paf_dev ends with one copy of max_humans-sized records
+ * into pinned host memory, which the host readers (ekp_results, ekp_results_humans) then read without touching the
+ * device.  enable == 0: batches submitted from now on leave the records on the device only.  That suits a caller who
+ * reads results only on the device (ekp_results_device*, ekp_draw_humans) and saves the copy on every batch (about
+ * 0.75 MB for 64 images at max_humans 32).  The host readers still work after such a run: the first of them waits for
+ * it and downloads its records once.  The mode is recorded with each run, so changing it does not affect a run
+ * already submitted, and each mode replays its own CUDA graph.  The process_paf surface is not affected. */
+int ekp_set_host_copy(ekp_ctx *ctx, int enable);
 
 /* ---- drawing (SURVEY.md 8f row f2) --------------------------------------------------------------
  * Paints the people of the last run onto n DEVICE frames uint8 [n, H, W, 3] (contiguous, in place), as the reference's

@@ -43,6 +43,10 @@ class DeviceResults(C.Structure):  # ekp_device_results: device pointers, None =
                 ("parts", C.c_void_p), ("scores", C.c_void_p)]
 
 
+class DevicePeaks(C.Structure):  # ekp_device_peaks: device pointers, None = that table is not written
+    _fields_ = [("n_peaks", C.c_void_p), ("peaks", C.c_void_p), ("part_off", C.c_void_p)]
+
+
 # every symbol include/ekpose_b200.h declares: (restype, argtypes)
 _vp, _i, _f = C.c_void_p, C.c_int, C.c_float
 SIGNATURES = {
@@ -59,6 +63,8 @@ SIGNATURES = {
     "ekp_results": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "ekp_results_humans": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "ekp_results_device": (_i, [_vp, _i, C.POINTER(DeviceResults), _vp]),
+    "ekp_results_device_peaks": (_i, [_vp, _i, C.POINTER(DevicePeaks), _vp]),
+    "ekp_set_host_copy": (_i, [_vp, _i]),
     "ekp_scipy_gauss3_weights": (_i, [_vp]),
     "ekp_debug_std_sort": (_i, [_vp, _vp, _vp, _i, _vp]),
     "ekp_results_parts": (_i, [_vp, _vp]),

@@ -11,6 +11,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <initializer_list>
 #include <vector>
 
 #include "capi.cuh"
@@ -310,7 +311,7 @@ int run_peak_sort(ekp_ctx* c, int n, int id_from_key, cudaStream_t st) {
     c->launches += 1;
     return EKP_OK;
 }
-int run_connect_assemble(ekp_ctx* c, int n, const PafSource& paf, int h1, cudaStream_t st, unsigned char* records_direct) {
+int run_connect_assemble(ekp_ctx* c, int n, const PafSource& paf, int h1, cudaStream_t st, bool host_copy, unsigned char* records_direct) {
     mark(c, 2, st);
     AsmParams ap;
     ap.line = c->line; ap.max_peaks = c->max_peaks; ap.n_peaks = c->n_peaks; ap.part_off = c->part_off; ap.conns = c->conns;
@@ -326,7 +327,7 @@ int run_connect_assemble(ekp_ctx* c, int n, const PafSource& paf, int h1, cudaSt
     mark(c, 4, st);
     if (c->timing) c->timed_runs++;
     c->launches += 2;
-    if (!records_direct) CU(cudaMemcpyAsync(c->h_records, c->records, c->lay.stride * (size_t) n, cudaMemcpyDeviceToHost, st));  // one packed copy
+    if (!records_direct && host_copy) CU(cudaMemcpyAsync(c->h_records, c->records, c->lay.stride * (size_t) n, cudaMemcpyDeviceToHost, st));  // one packed copy
     return EKP_OK;
 }
 PafSource paf_source(int mode, const void* ptr, const int* pair_base, int f1, int f2, int f3) {
@@ -335,20 +336,20 @@ PafSource paf_source(int mode, const void* ptr, const int* pair_base, int f1, in
     s.layout = EKP_LAYOUT_NHWC; s.H = f1; s.W = f2; s.C = f3; s.h = f1 / 8; s.w = f2 / 8;
     return s;
 }
-int finish_submit(ekp_ctx* c, int n, cudaStream_t st) {
+int finish_submit(ekp_ctx* c, int n, cudaStream_t st, bool records_on_host) {
     CU(cudaEventRecord(c->done, st));
-    c->last_stream = st; c->last_n = n; c->has_run = true;
+    c->last_stream = st; c->last_n = n; c->has_run = true; c->records_on_host = records_on_host;
     return EKP_OK;
 }
-static int run_back_half(ekp_ctx* c, int n, int id_from_key, const PafSource& paf, int h1, cudaStream_t st) {
+static int run_back_half(ekp_ctx* c, int n, int id_from_key, const PafSource& paf, int h1, cudaStream_t st, bool host_copy) {
     int rc = run_peak_sort(c, n, id_from_key, st);
     if (rc) return rc;
-    return run_connect_assemble(c, n, paf, h1, st);
+    return run_connect_assemble(c, n, paf, h1, st, host_copy);
 }
 
 // ---- one batch, stages 1-5 ------------------------------------------------------------------------------------
-// Everything one batch puts on a stream: input copies (host entry), counters, the kernels of stages 1-5 and the one packed
-// device-to-host copy of the result records.  Issued eagerly or into a stream capture.
+// Everything one batch puts on a stream: input copies (host entry), counters, the kernels of stages 1-5 and, in host-copy
+// mode, the one packed device-to-host copy of the result records.  Issued eagerly or into a stream capture.
 static int enqueue_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
     const bool wide = a.dtype == EKP_DTYPE_F32;
     if (a.heat_host) {
@@ -394,14 +395,14 @@ static int enqueue_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
         if (a.heat_mat) { CU(launch_upsample_nearest(a.heat, a.layout, a.n, a.h, a.w, EKP_HEAT_CH, a.heat_mat, st)); c->launches += 1; }
         src.ptr = a.paf; src.mode = PAF_LO_NEAREST;  // == paf_mat[y][x] exactly (cv2 INTER_NEAREST x8)
     }
-    return run_back_half(c, a.n, /*id_from_key=*/0, src, /*h1=*/8 * a.h, st);
+    return run_back_half(c, a.n, /*id_from_key=*/0, src, /*h1=*/8 * a.h, st, a.host_copy != 0);
 }
 
 static bool same_args(const PostArgs& a, const PostArgs& b) {
     return a.heat == b.heat && a.paf == b.paf && a.heat_host == b.heat_host && a.paf_host == b.paf_host && a.heat16 == b.heat16 &&
            a.paf16 == b.paf16 && a.dtype == b.dtype && a.n == b.n && a.h == b.h &&
            a.w == b.w && a.layout == b.layout && a.frontend == b.frontend && memcmp(&a.thr, &b.thr, sizeof(float)) == 0 &&
-           a.heat_mat == b.heat_mat && a.paf_mat == b.paf_mat;
+           a.heat_mat == b.heat_mat && a.paf_mat == b.paf_mat && a.host_copy == b.host_copy;
 }
 
 // A context keeps the graphs of its last kMaxGraphs keys, the least recently used one evicted first: a stream of frames
@@ -468,7 +469,7 @@ static int submit_batch(ekp_ctx* c, const PostArgs& a, cudaStream_t st) {
     rc = launch_cached(c, key, epoch, st, [&](cudaStream_t q) { return enqueue_batch(c, a, q); });
     if (rc) return rc;
     c->map_h = 8 * a.h; c->map_w = 8 * a.w;
-    return finish_submit(c, a.n, st);
+    return finish_submit(c, a.n, st, a.host_copy != 0);
 }
 
 // the context's float32 input block [heat | paf] (host entry: the copy target; 16-bit inputs: the widening target)
@@ -493,6 +494,7 @@ static int post_args(const ekp_ctx* c, const void* heat, const void* paf, int dt
         return fail(EKP_ERR_ARG, "%s: 16-bit heat / paf must be 2-byte aligned", who);
     *a = PostArgs{};
     a->dtype = dtype; a->n = n; a->h = h; a->w = w; a->layout = layout; a->frontend = frontend; a->thr = thr_heat;
+    a->host_copy = c->host_copy;
     return EKP_OK;
 }
 
@@ -585,17 +587,25 @@ extern "C" int ekp_process_paf_dev(ekp_ctx* c, const float* peaks, const int* n_
     mark(c, 0, st);
     CU(launch_peaks_ingest(peaks, n_peaks, 0, peaks_stride, 5, n, W, H, c->raw, c->raw_count, c->max_peaks, c->overflow, st));
     c->launches += 1;
-    int rc = run_back_half(c, n, /*id_from_key=*/1, paf_source(PAF_FULL_HWC, paf_mat, nullptr, H, W, C), h1, st);
+    const bool host_copy = c->host_copy;
+    int rc = run_back_half(c, n, /*id_from_key=*/1, paf_source(PAF_FULL_HWC, paf_mat, nullptr, H, W, C), h1, st, host_copy);
     if (rc) return rc;
     c->map_h = H; c->map_w = W;
-    return finish_submit(c, n, st);
+    return finish_submit(c, n, st, host_copy);
 }
 
-static int wait_results(ekp_ctx* c, const char* who) {
+// Waits for the last run.  records: the caller reads the records in h_records, so a run that left them on the device only
+// (ekp_set_host_copy(ctx, 0)) has them downloaded here, once per run.
+static int wait_results(ekp_ctx* c, const char* who, bool records) {
     if (!c) return fail(EKP_ERR_ARG, "%s: NULL context", who);
     if (!c->has_run) return fail(EKP_ERR_STATE, "%s: no run has been submitted on this context", who);
     CU(cudaSetDevice(c->device));
     CU(cudaEventSynchronize(c->done));
+    if (records && !c->records_on_host) {
+        CU(cudaMemcpyAsync(c->h_records, c->last_records, c->lay.stride * (size_t) c->last_n, cudaMemcpyDeviceToHost, c->last_stream));
+        CU(cudaStreamSynchronize(c->last_stream));
+        c->records_on_host = true;
+    }
     return EKP_OK;
 }
 struct RecHead { int num_humans, n_peaks; unsigned overflow; int pad; };
@@ -611,7 +621,7 @@ static int overflow_status(const ekp_ctx* c) {
 }
 
 extern "C" int ekp_results(ekp_ctx* c, int* num_humans, float* subset, int* n_peaks, ekp_peak* peaks_line, unsigned* overflow) {
-    int rc = wait_results(c, "ekp_results");
+    int rc = wait_results(c, "ekp_results", true);
     if (rc) return rc;
     const int n = c->last_n;
     const size_t mh = (size_t) c->max_humans;
@@ -634,7 +644,7 @@ extern "C" int ekp_results(ekp_ctx* c, int* num_humans, float* subset, int* n_pe
 }
 
 extern "C" int ekp_results_humans(ekp_ctx* c, int* num_humans, ekp_peak* parts, float* scores, unsigned* overflow) {
-    int rc = wait_results(c, "ekp_results_humans");
+    int rc = wait_results(c, "ekp_results_humans", true);
     if (rc) return rc;
     const int n = c->last_n;
     const size_t mh = (size_t) c->max_humans;
@@ -690,23 +700,50 @@ extern "C" int ekp_draw_humans(ekp_ctx* c, unsigned char* frames, int n, int H, 
     });
 }
 
+// The checks ekp_results_device and ekp_results_device_peaks share, after the NULL context / out check.  *any: a table is
+// to be written.
+static int export_args(const ekp_ctx* c, int n, std::initializer_list<const void*> ptrs, const char* who, bool* any) {
+    if (!c->has_run) return fail(EKP_ERR_STATE, "%s: no run has been submitted on this context", who);
+    if (n != c->last_n) return fail(EKP_ERR_ARG, "%s: tables for %d images, the run had %d", who, n, c->last_n);
+    *any = false;
+    for (const void* p : ptrs) {
+        if (reinterpret_cast<uintptr_t>(p) & 3u) return fail(EKP_ERR_ARG, "%s: a pointer is not 4-byte aligned", who);
+        *any = *any || p;
+    }
+    return EKP_OK;
+}
+
 extern "C" int ekp_results_device(ekp_ctx* c, int n, const ekp_device_results* out, void* stream) {
     if (!c || !out) return fail(EKP_ERR_ARG, "ekp_results_device: NULL %s", c ? "out" : "context");
-    if (!c->has_run) return fail(EKP_ERR_STATE, "ekp_results_device: no run has been submitted on this context");
-    if (n != c->last_n) return fail(EKP_ERR_ARG, "ekp_results_device: tables for %d images, the run had %d", n, c->last_n);
-    const void* ptrs[] = {out->num_humans, out->overflow, out->n_peaks, out->subset, out->parts, out->scores};
     bool any = false;
-    for (const void* p : ptrs) {
-        if (reinterpret_cast<uintptr_t>(p) & 3u) return fail(EKP_ERR_ARG, "ekp_results_device: a pointer is not 4-byte aligned");
-        any = any || p;
-    }
-    if (!any) return EKP_OK;
+    int rc = export_args(c, n, {out->num_humans, out->overflow, out->n_peaks, out->subset, out->parts, out->scores},
+                         "ekp_results_device", &any);
+    if (rc || !any) return rc;
     cudaStream_t st = (cudaStream_t) stream;
     return after_run(c, st, [&]() {
         CU(launch_results_export(c->last_records, c->lay, c->max_humans, n, *out, st));
         c->launches += 1;
         return (int) EKP_OK;
     });
+}
+
+extern "C" int ekp_results_device_peaks(ekp_ctx* c, int n, const ekp_device_peaks* out, void* stream) {
+    if (!c || !out) return fail(EKP_ERR_ARG, "ekp_results_device_peaks: NULL %s", c ? "out" : "context");
+    bool any = false;
+    int rc = export_args(c, n, {out->n_peaks, out->peaks, out->part_off}, "ekp_results_device_peaks", &any);
+    if (rc || !any) return rc;
+    cudaStream_t st = (cudaStream_t) stream;
+    return after_run(c, st, [&]() {
+        CU(launch_peaks_export(c->last_records, c->lay.stride, c->line, c->part_off, c->max_peaks, n, *out, st));
+        c->launches += 1;
+        return (int) EKP_OK;
+    });
+}
+
+extern "C" int ekp_set_host_copy(ekp_ctx* c, int enable) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_set_host_copy: NULL context");
+    c->host_copy = enable != 0;
+    return EKP_OK;
 }
 
 extern "C" int ekp_debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask) {
@@ -813,7 +850,7 @@ extern "C" int ekp_set_timing(ekp_ctx* c, int enable) {
 }
 
 extern "C" int ekp_stage_times(ekp_ctx* c, float* ms, int* runs) {
-    int rc = wait_results(c, "ekp_stage_times");
+    int rc = wait_results(c, "ekp_stage_times", false);
     if (rc) return rc;
     if (!ms) return fail(EKP_ERR_ARG, "ekp_stage_times: NULL pointer");
     CU(cudaStreamSynchronize(c->last_stream));
@@ -831,7 +868,7 @@ extern "C" int ekp_stage_times(ekp_ctx* c, float* ms, int* runs) {
 }
 
 extern "C" int ekp_results_parts(ekp_ctx* c, int* part_off) {
-    int rc = wait_results(c, "ekp_results_parts");
+    int rc = wait_results(c, "ekp_results_parts", false);
     if (rc) return rc;
     if (!part_off) return fail(EKP_ERR_ARG, "ekp_results_parts: NULL pointer");
     std::vector<int> tmp((size_t) c->last_n * 20);

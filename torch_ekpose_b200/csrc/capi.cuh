@@ -44,6 +44,8 @@ cudaError_t launch_draw(const unsigned char* records, const ResultLayout& lay, i
                         unsigned char* frames, int n, int H, int W, unsigned* keys, unsigned epoch, cudaStream_t stream);
 cudaError_t launch_results_export(const unsigned char* records, const ResultLayout& lay, int max_humans, int n,
                                   const ekp_device_results& out, cudaStream_t stream);
+cudaError_t launch_peaks_export(const unsigned char* records, size_t stride, const ekp_peak* line, const int* part_off, int max_peaks,
+                                int n, const ekp_device_peaks& out, cudaStream_t stream);
 void debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask);
 void debug_draw_host(const int* num_humans, const ekp_peak* parts, int max_humans, int map_h, int map_w,
                      unsigned char* frames, int n, int H, int W);
@@ -60,6 +62,7 @@ struct PostArgs {
     int n, h, w, layout, frontend;
     float thr;
     float *heat_mat, *paf_mat;
+    int host_copy;                      // the batch ends with the device-to-host copy of its records (ekp_set_host_copy)
 };
 
 // What a cached CUDA graph was captured for.  A batch of the context API is keyed by its arguments; process_paf's
@@ -88,6 +91,8 @@ struct ekp_ctx {
     int* n_conns = nullptr;         // [max_batch][19]
     unsigned char* records = nullptr;  // [max_batch] packed result records (ResultLayout)
     const unsigned char* last_records = nullptr;  // where the last run's assembly wrote them (records, or pinned host)
+    bool host_copy = true;          // batches submitted from now on copy their records to h_records (ekp_set_host_copy)
+    bool records_on_host = false;   // h_records holds the last run's records (else wait_results downloads them first)
     int map_h = 0, map_w = 0;       // the last run's full-resolution map, by which ekp_draw_humans normalises
     unsigned* draw_keys = nullptr;  // ekp_draw_humans' per-pixel keys (lazily, grown on demand)
     size_t draw_keys_cap = 0;       // pixels
@@ -144,13 +149,16 @@ int fail(int code, const char* fmt, ...);
 
 // stages 4-5 + result copies, shared by every entry point; each adds the kernels it launches to c->launches
 int run_peak_sort(ekp_ctx* c, int n, int id_from_key, cudaStream_t st);
-// records_direct: device-visible pinned host memory the assembly writes the result records to itself (no D2H copy node)
-int run_connect_assemble(ekp_ctx* c, int n, const ekp::PafSource& paf, int h1, cudaStream_t st, unsigned char* records_direct = nullptr);
+// host_copy: end with the one device-to-host copy of the result records into h_records.  records_direct: device-visible
+// pinned host memory the assembly writes the result records to itself (no copy node, host_copy is ignored).
+int run_connect_assemble(ekp_ctx* c, int n, const ekp::PafSource& paf, int h1, cudaStream_t st, bool host_copy,
+                         unsigned char* records_direct = nullptr);
 // Stage 4's view of a caller's paf_mat [f1][f2][f3] (NHWC), in which a peak's id is its row in the caller's peak table: the
 // tensor itself (PAF_FULL_HWC) or the samples gathered from it (PAF_PACKED, laid out by pair_base).
 ekp::PafSource paf_source(int mode, const void* ptr, const int* pair_base, int f1, int f2, int f3);
-// after a run has been put on `st` (eagerly or as a graph launch): results become readable when `done` fires
-int finish_submit(ekp_ctx* c, int n, cudaStream_t st);
+// after a run has been put on `st` (eagerly or as a graph launch): results become readable when `done` fires.
+// records_on_host: the run leaves its records in h_records (a copy or the direct write-out), else only on the device.
+int finish_submit(ekp_ctx* c, int n, cudaStream_t st, bool records_on_host);
 
 // Puts on `st` what enqueue(q) issues on a stream q, as a replay of the context's CUDA graph for `key`: captured and
 // instantiated on the first use of the key, then one launch call instead of many stream operations, and no gaps

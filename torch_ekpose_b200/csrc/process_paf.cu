@@ -211,7 +211,7 @@ int process_paf_listed(ekp_ctx* c, long long npk, int p3, const float* peaks, in
             int rc = ingest_and_sort(c, blk_peaks, (int) npk, p3, f1, f2, q);
             if (rc) return rc;
         }
-        return run_connect_assemble(c, 1, src, h1, q, zero_copy ? c->h_records_dev : nullptr);
+        return run_connect_assemble(c, 1, src, h1, q, /*host_copy=*/true, zero_copy ? c->h_records_dev : nullptr);
     };
     const cudaStream_t st = nullptr;
     if (zero_copy) return launch_cached(c, GraphKey{{}, {p3, f1, f2, f3, h1, (long long) bytes}}, 0, st, enqueue);
@@ -263,12 +263,12 @@ int process_paf_uploaded(ekp_ctx* c, long long npk, int p3, const float* peaks, 
             g_host_samp[k] = make_float2(q[0], q[1]);
         }
         CU(cudaMemcpyAsync(g_dev_samp, g_host_samp, ns * sizeof(float2), cudaMemcpyHostToDevice, st));
-        return run_connect_assemble(c, 1, paf_source(PAF_PACKED, g_dev_samp, g_dev_pair_base, f1, f2, f3), h1, st);
+        return run_connect_assemble(c, 1, paf_source(PAF_PACKED, g_dev_samp, g_dev_pair_base, f1, f2, f3), h1, st, /*host_copy=*/true);
     }
     rc = grow(g_dev_paf, g_dev_paf_cap, paf_elems);
     if (rc) return rc;
     CU(cudaMemcpyAsync(g_dev_paf, pafmap, paf_elems * sizeof(float), cudaMemcpyHostToDevice, st));
-    return run_connect_assemble(c, 1, paf_source(PAF_FULL_HWC, g_dev_paf, nullptr, f1, f2, f3), h1, st);
+    return run_connect_assemble(c, 1, paf_source(PAF_FULL_HWC, g_dev_paf, nullptr, f1, f2, f3), h1, st, /*host_copy=*/true);
 }
 
 // the getters' view of a finished run
@@ -305,7 +305,7 @@ extern "C" int process_paf(int p1, int p2, int p3, float* peaks, int h1, int h2,
         rc = offsets_fit && (!route || strcmp(route, "listed") == 0) ? process_paf_listed(c, npk, p3, peaks, h1, f1, f2, f3, pafmap, line) : 1;
         const bool listed = rc == EKP_OK;
         if (rc == 1) rc = process_paf_uploaded(c, npk, p3, peaks, h1, f1, f2, f3, pafmap, offsets_fit && !(route && strcmp(route, "dense") == 0));
-        if (rc == EKP_OK) rc = finish_submit(c, 1, nullptr);
+        if (rc == EKP_OK) rc = finish_submit(c, 1, nullptr, /*records_on_host=*/true);
         if (rc) return rc;
         std::vector<float> subset((size_t) c->max_humans * 20);
         int nh = 0, np = 0;

@@ -1,5 +1,6 @@
-// results_device.cu -- the last run's result tables written into caller-owned DEVICE buffers (ekp_results_device): the
-// device counterpart of ekp_results / ekp_results_humans, ordered on a stream after the run, with no host wait.
+// results_device.cu -- the last run's result tables written into caller-owned DEVICE buffers (ekp_results_device, and
+// ekp_results_device_peaks for the peak table): the device counterpart of ekp_results / ekp_results_humans /
+// ekp_results_parts, ordered on a stream after the run, with no host wait.
 //
 // Each image's packed record (ResultLayout) holds the header, then the subset rows, the per-human part table and the
 // human scores, every region starting on a 16-byte boundary.  Rows below min(num_humans, max_humans) are copied byte for
@@ -90,6 +91,49 @@ cudaError_t launch_results_export(const unsigned char* records, const ResultLayo
     const int kThreads = 256, kUnitsPerThread = 2;
     const unsigned chunks = (unsigned) ((units + kThreads * kUnitsPerThread - 1) / (kThreads * kUnitsPerThread));
     results_export_kernel<<<dim3(chunks, (unsigned) n), kThreads, 0, stream>>>(P);
+    return cudaGetLastError();
+}
+
+// ---- the peak table (ekp_results_device_peaks) -------------------------------------------------------------------------
+// The context's part-sorted table line [n][max_peaks] and part_off [n][20] (the 20th entry is not exported), with each
+// image's peak count taken from its record header as the host reader takes it.  Rows from min(n_peaks, max_peaks) on
+// are written as zero bytes, like the people's padding above.
+struct PeaksExportParams {
+    const unsigned char* records;
+    size_t stride;
+    const unsigned* line;      // ekp_peak [n][max_peaks] as words
+    const unsigned* part_off;  // [n][20]
+    int max_peaks;
+    int* n_peaks;
+    unsigned* peaks;           // [n][max_peaks * 4] or nullptr
+    int* part_off_out;         // [n][19] or nullptr
+    bool vec;                  // peaks is 16-byte aligned (every image's table then is)
+};
+
+__global__ void __launch_bounds__(256) peaks_export_kernel(const PeaksExportParams P) {
+    const int img = blockIdx.y;
+    const int npk = reinterpret_cast<const int4*>(P.records + P.stride * (size_t) img)->y;  // num_humans, n_peaks, overflow, pad
+    if (blockIdx.x == 0 && threadIdx.x == 0 && P.n_peaks) P.n_peaks[img] = npk;
+    const int first = blockIdx.x * blockDim.x + threadIdx.x, step = gridDim.x * blockDim.x;
+    const int total = 4 * P.max_peaks;
+    if (P.peaks)
+        copy_region(P.line + (size_t) img * total, P.peaks + (size_t) img * total, 4 * min(npk, P.max_peaks), total, P.vec, first, step);
+    if (P.part_off_out)
+        copy_region(P.part_off + (size_t) img * 20, reinterpret_cast<unsigned*>(P.part_off_out) + (size_t) img * 19, 19, 19, false,
+                    first, step);
+}
+
+cudaError_t launch_peaks_export(const unsigned char* records, size_t stride, const ekp_peak* line, const int* part_off, int max_peaks,
+                                int n, const ekp_device_peaks& out, cudaStream_t stream) {
+    PeaksExportParams P;
+    P.records = records; P.stride = stride; P.max_peaks = max_peaks;
+    P.line = reinterpret_cast<const unsigned*>(line); P.part_off = reinterpret_cast<const unsigned*>(part_off);
+    P.n_peaks = out.n_peaks; P.peaks = reinterpret_cast<unsigned*>(out.peaks); P.part_off_out = out.part_off;
+    P.vec = (reinterpret_cast<uintptr_t>(out.peaks) & 15u) == 0;
+    const int units = out.peaks ? (P.vec ? max_peaks : 4 * max_peaks) : 19;
+    const int kThreads = 256, kUnitsPerThread = 2;
+    const unsigned chunks = (unsigned) ((units + kThreads * kUnitsPerThread - 1) / (kThreads * kUnitsPerThread));
+    peaks_export_kernel<<<dim3(chunks, (unsigned) n), kThreads, 0, stream>>>(P);
     return cudaGetLastError();
 }
 

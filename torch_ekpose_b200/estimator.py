@@ -13,7 +13,8 @@ stay on the device in the layout it emits (NCHW): no device-to-host copy, no tra
 ``infer_humans`` feeds them straight to the CUDA post-processing on the same device, and
 ``infer_and_draw`` also paints the people onto the uploaded frames (``ekp_draw_humans``, byte for
 byte the reference's ``draw_humans``), and ``infer_human_tensors`` returns the people as CUDA tensors
-(``ekp_results_device``) without waiting for the device.  There is no host implementation of any of this in the
+(``ekp_results_device``) without waiting for the device; these two leave the result records on the device (no
+per-batch copy to the host, ``ekp_set_host_copy``).  There is no host implementation of any of this in the
 package; the model itself is the caller's (cuDNN through PyTorch; out of scope).
 """
 from __future__ import annotations
@@ -72,7 +73,10 @@ def get_outputs_batched(images, model, preprocess: str, device):
     return _forward(_upload(images, idx), model, preprocess, idx)
 
 
-def _postprocess(heats, pafs, frontend: str, thr: float) -> PostProcessor:
+def _postprocess(heats, pafs, frontend: str, thr: float, host_copy: bool) -> PostProcessor:
+    """host_copy: the caller reads the people on the host (the run then ends with the copy of its records there); the
+    device-only callers leave them on the device.  The mode is set per call because the context is shared, and each
+    mode replays its own CUDA graph."""
     n, _, h, w = heats.shape
     idx = heats.device.index
     key = (idx, n, h, w)
@@ -80,6 +84,7 @@ def _postprocess(heats, pafs, frontend: str, thr: float) -> PostProcessor:
     if pp is None:
         pp = _pp_cache[key] = PostProcessor(device=idx, max_batch=n, max_h=h, max_w=w, max_peaks=2048, max_humans=128)
     _last_pp[0] = pp
+    pp.set_host_copy(host_copy)
     pp.run(heats, pafs, layout="nchw", frontend=frontend, thr=thr)   # bf16 / fp16 under autocast: widened on the device
     return pp
 
@@ -90,28 +95,31 @@ def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, f
     (the network's outputs never leave the device, and 16-bit outputs of a model under torch.autocast are taken as
     they are).  ``frontend='reference'`` gives the reference's people."""
     pafs, heats, _ = get_outputs_batched(images, model, preprocess, device)
-    return _postprocess(heats, pafs, frontend, thr).humans()
+    return _postprocess(heats, pafs, frontend, thr, True).humans()
 
 
 def infer_human_tensors(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15,
-                        subset: bool = False):
+                        subset: bool = False, peaks: bool = False):
     """``infer_humans`` with the people left on the GPU: returns (tensors, im_scale), ``tensors`` being the dict of
     CUDA tensors ``PostProcessor.result_tensors(subset=subset)`` returns (per image num_humans, overflow, n_peaks,
-    the part table, part and human scores) and ``im_scale`` that of ``get_outputs_batched``.  Nothing waits for the
-    device and nothing raises on a capacity overflow: the caller checks ``tensors['overflow']``."""
+    the part table, part and human scores; with ``peaks=True`` also the peak table) and ``im_scale`` that of
+    ``get_outputs_batched``.  Nothing waits for the device and nothing raises on a capacity overflow: the caller checks
+    ``tensors['overflow']``.  The batch leaves its records on the device (no copy to the host); ``last_postprocessor()``'s
+    host readers still work, at the cost of one download."""
     pafs, heats, im_scale = get_outputs_batched(images, model, preprocess, device)
-    return _postprocess(heats, pafs, frontend, thr).result_tensors(subset=subset), im_scale
+    return _postprocess(heats, pafs, frontend, thr, False).result_tensors(subset=subset, peaks=peaks), im_scale
 
 
 def infer_and_draw(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15):
     """``infer_humans`` followed by the reference's ``draw_humans`` on every frame, all on the GPU: returns the drawn
     frames, a CUDA uint8 tensor [n,H,W,3] on ``device``.  Host frames are drawn on the copy uploaded for the
     preprocessing; a CUDA tensor on ``device`` (contiguous) is drawn in place.  The people stay available through
-    ``last_postprocessor()``; the call does not wait for the device."""
+    ``last_postprocessor()`` (the batch leaves its records on the device: its first host reader downloads them); the
+    call does not wait for the device."""
     idx = _device_index(device)
     frames = _upload(images, idx)
     pafs, heats, _ = _forward(frames, model, preprocess, idx)
-    return _postprocess(heats, pafs, frontend, thr).draw_humans(frames)
+    return _postprocess(heats, pafs, frontend, thr, False).draw_humans(frames)
 
 
 def last_postprocessor():

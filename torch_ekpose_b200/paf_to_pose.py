@@ -72,6 +72,7 @@ class PostProcessor:
         self.max_batch, self.max_h, self.max_w = max_batch, max_h, max_w
         self.max_peaks, self.max_humans = max_peaks, max_humans
         self.max_part, self.max_cand = int(_lib.lib.ekp_max_part(self._ctx)), int(_lib.lib.ekp_max_cand(self._ctx))
+        self.host_copy = True  # ekp_set_host_copy
         self._keep = None      # inputs of the in-flight run
         self._n = 0
         self._hw = (0, 0)
@@ -217,15 +218,25 @@ class PostProcessor:
         _lib.check(_lib.lib.ekp_results_humans(self._ctx, num.ctypes.data, parts.ctypes.data, scores.ctypes.data, None))
         return num, parts, scores
 
-    def _result_specs(self, n: int, subset: bool):
+    def set_host_copy(self, enable: bool) -> None:
+        """Whether the batches submitted from now on end with the device-to-host copy of their result records (the
+        default: on).  Off suits a caller who reads the results only on the device (``result_tensors``,
+        ``draw_humans``) and saves the copy on every batch; ``results`` / ``human_tables`` / ``humans`` still work
+        after such a run (the first of them downloads the records)."""
+        _lib.check(_lib.lib.ekp_set_host_copy(self._ctx, int(bool(enable))))
+        self.host_copy = bool(enable)
+
+    def _result_specs(self, n: int, subset: bool, peaks: bool):
         mh = self.max_humans
         specs = [("num_humans", (n,), torch.int32), ("overflow", (n,), torch.int32), ("n_peaks", (n,), torch.int32),
                  ("parts", (n, mh, _lib.NUM_PART, 4), torch.int32), ("scores", (n, mh), torch.float32)]
         if subset:
             specs.append(("subset", (n, mh, _lib.SUBSET_COLS), torch.float32))
+        if peaks:
+            specs += [("peaks", (n, self.max_peaks, 4), torch.int32), ("part_off", (n, _lib.NUM_PART + 1), torch.int32)]
         return specs
 
-    def result_tensors(self, *, subset: bool = False, out: Optional[dict] = None, stream=None) -> dict:
+    def result_tensors(self, *, subset: bool = False, peaks: bool = False, out: Optional[dict] = None, stream=None) -> dict:
         """The tables of the last run as CUDA tensors on this context's device, without waiting for the device: the
         export is one kernel on ``stream`` (default: the current stream), ordered after the run and before this
         context's next run on any stream.
@@ -234,7 +245,10 @@ class PostProcessor:
         ``parts`` int32 [n, max_humans, 18, 4] (x, y, score bits, id; id -1 = absent, as ``human_tables``),
         ``part_score`` float32 [n, max_humans, 18] (the view ``parts[..., 2].view(torch.float32)``), ``scores``
         float32 [n, max_humans] and, with ``subset=True``, ``subset`` float32 [n, max_humans, 20] (as ``results``).
-        Rows from ``num_humans[i]`` on are zero, so each tensor copied to the host equals the host table byte for byte.
+        ``peaks=True`` adds the part-sorted peak table of ``results(with_peaks=True)``: ``peaks`` int32
+        [n, max_peaks, 4] (x, y, score bits, id), its ``peak_score`` float32 view and ``part_off`` int32 [n, 19].
+        Rows from ``num_humans[i]`` (people) and ``n_peaks[i]`` (peaks) on are zero, so each tensor copied to the host
+        equals the host table byte for byte.
 
         This never raises on a capacity overflow (nothing is known about it when the call returns): the caller checks
         ``overflow``, where a non-zero entry means that image's tables were cut.  New tensors are allocated under the
@@ -245,7 +259,7 @@ class PostProcessor:
         if not n:
             raise _lib.EkpError(_lib.ERR_STATE, "result_tensors: no run has been submitted on this context")
         dev = torch.device("cuda", self.device)
-        specs = self._result_specs(n, subset)
+        specs = self._result_specs(n, subset, peaks)
         if out is None:
             if stream is None:
                 st = torch.cuda.current_stream(dev)
@@ -263,8 +277,13 @@ class PostProcessor:
                     raise ValueError(f"out[{name!r}] must be a contiguous {dt} tensor {list(shape)} on {dev}")
         tabs = _lib.DeviceResults(*(out[k].data_ptr() if k in out and (k != "subset" or subset) else None
                                     for k in ("num_humans", "overflow", "n_peaks", "subset", "parts", "scores")))
-        _lib.check(_lib.lib.ekp_results_device(self._ctx, n, C.byref(tabs), self._stream(stream)))
+        st = self._stream(stream)
+        _lib.check(_lib.lib.ekp_results_device(self._ctx, n, C.byref(tabs), st))
         out["part_score"] = out["parts"][..., 2].view(torch.float32)
+        if peaks:   # n_peaks came with the people
+            pk = _lib.DevicePeaks(None, out["peaks"].data_ptr(), out["part_off"].data_ptr())
+            _lib.check(_lib.lib.ekp_results_device_peaks(self._ctx, n, C.byref(pk), st))
+            out["peak_score"] = out["peaks"][..., 2].view(torch.float32)
         return out
 
     def humans(self) -> List[List[Human]]:
@@ -428,6 +447,7 @@ def _processor(device: int, n: int, h: int, w: int, max_peaks: int, max_humans: 
             pp.close()
         raise
     if pp is not None:
+        new.set_host_copy(pp.host_copy)   # the grown context keeps the caller's mode
         pp.close()
     _cache[key] = new
     return new
