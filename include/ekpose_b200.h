@@ -20,7 +20,8 @@
  *    batch goes from the network's stride-8 outputs to people in one call.  The people come back as host tables
  *    (ekp_results, ekp_results_humans: these wait for the run) or into caller-owned device buffers, ordered on a
  *    stream with no host wait (ekp_results_device, ekp_results_device_peaks).  A caller that reads them only on the
- *    device can also skip each batch's copy of the result records to the host (ekp_set_host_copy).
+ *    device can also skip each batch's copy of the result records to the host (ekp_set_host_copy), and give its people
+ *    stable ids across video frames on the device (ekp_track_humans).
  *
  * All functions return EKP_OK (0) or a negative ekp_status; ekp_last_error() returns a
  * thread-local human-readable message for the last failure.  Nothing aborts.
@@ -213,6 +214,55 @@ int ekp_results_device_peaks(ekp_ctx *ctx, int n, const ekp_device_peaks *out, v
  * it and downloads its records once.  The mode is recorded with each run, so changing it does not affect a run
  * already submitted, and each mode replays its own CUDA graph.  The process_paf surface is not affected. */
 int ekp_set_host_copy(ekp_ctx *ctx, int enable);
+
+/* ---- tracking: stable person ids across video frames ----------------------------------------------------------------
+ * Gives every person of a frame the id of the same person in earlier frames of its sequence, from the device human
+ * tables (ekp_results_device's num_humans and parts), so a video caller keeps the people on the GPU from frame to id.
+ * A call takes the tables of n images and n_seq sequences (n % n_seq == 0, F = n / n_seq): image i is frame i % F of
+ * sequence i / F.  n_seq = 1 is a batch of consecutive frames of one video, F = 1 is n_seq cameras with one frame each.
+ * Each sequence keeps its own tracks, frame counter and next id (ids start at 0 and grow by 1 per new track) in `state`,
+ * across calls.  The people of image i are rows 0 .. min(num_humans[i], max_humans) - 1 of parts [n, max_humans, 18]
+ * (overflow or not: the table is tracked as it stands).
+ *   similarity  COCO's OKS in float64 against the track's last pose: keypoint j = reference part ORDER_COCO[j]
+ *               (torch_ekpose_b200/coco.py; the neck is not used), pycocotools' sigmas / 10 and vars = (2 sigma)^2,
+ *               area = the integer (xmax - xmin + 1) * (ymax - ymin + 1) of the track's present keypoints, and over the m
+ *               keypoints present in both, in order of j, e_j = d2_j / var_j / area / 2 (d2_j = dx*dx + dy*dy, exact):
+ *               sim = sum of exp(-e_j) / m, or 0 when m == 0.
+ *   matching    per frame, the pairs (person, live track) with sim >= (double) min_oks, in descending sim, then
+ *               ascending track id, then ascending row; a pair is accepted when neither side is taken.  A matched person
+ *               gets its track's id, and the track its whole pose.  Unmatched people open new tracks in row order.
+ *   age         a track last matched at frame f0 can be matched at frames f0 + 1 .. f0 + max_age + 1, then is dropped.
+ *   capacity    a new track that finds all max_tracks slots live takes the slot of the track with the smallest last
+ *               match frame, then the smallest id, among those neither matched nor opened in this frame.
+ * ids int32 [n, max_humans] gets each row's track id, and -1 from row num_humans[i] on.
+ * Every pointer is a caller-owned DEVICE pointer: the tables and ids 4-byte aligned, the state 8-byte aligned.  The
+ * state's layout is private; its size depends only on (n_seq, max_tracks), so it outlives any context (a context
+ * re-created with larger capacities keeps tracking on the same state).  It holds the track poses and, per sequence, a
+ * max_tracks x max_tracks scratch of similarities for frames whose pairs do not fit shared memory.  Poses are kept in
+ * the map pixels of the runs that produced them: feeding one sequence runs of a different map size is the caller's
+ * error.  Frame counters are 32-bit.
+ * ekp_track_humans is one kernel launch (one block per sequence, counted in ekp_kernel_launches, not part of any batch
+ * graph), asynchronous on `stream`; it never waits on the host and never allocates.  The context only supplies the
+ * device and the error reporting: the call reads the caller's tables, not the context's records, so it composes with
+ * ekp_results_device on the same stream, and ordering across streams is the caller's.  EKP_ERR_ARG for a NULL pointer,
+ * n < 1 or n % n_seq != 0, max_humans outside [1, max_tracks], max_tracks outside [1, EKP_LIMIT_TRACKS], max_age < 0, a
+ * negative or non-finite min_oks, or a misaligned pointer. */
+#define EKP_LIMIT_TRACKS 512   /* slots of one sequence: at max_humans = max_tracks = 512 the per-block working set
+                                * (tracks, the frame's people, lists) takes 172,192 of the 232,448 bytes of shared memory
+                                * of one block, and the rest holds the similarity matrix */
+/* Bytes of a state for n_seq sequences of up to max_tracks tracks; 0 when n_seq < 1 or max_tracks is outside
+ * [1, EKP_LIMIT_TRACKS].  long long rather than size_t: every function of this header returns int, float, long long,
+ * void or a pointer, the set tests/test_abi.py parses to check the header against the library and its Python binding;
+ * the value is a non-negative byte count. */
+long long ekp_track_state_bytes(int n_seq, int max_tracks);
+/* Clears a state asynchronously on `stream` (cudaMemsetAsync): no tracks, frame 0, next id 0 in every sequence. */
+int ekp_track_reset(ekp_ctx *ctx, void *state, int n_seq, int max_tracks, void *stream);
+int ekp_track_humans(ekp_ctx *ctx, const int *num_humans, const ekp_peak *parts, int n, int max_humans, void *state,
+                     int n_seq, int max_tracks, float min_oks, int max_age, int *ids, void *stream);
+/* Test hook for ekp_track_humans: the same code, run serially on the CPU on HOST buffers (and a host state), with the same
+ * arguments and checks.  It is not a CPU path of the tracker. */
+int ekp_debug_track_host(const int *num_humans, const ekp_peak *parts, int n, int max_humans, void *state, int n_seq,
+                         int max_tracks, float min_oks, int max_age, int *ids);
 
 /* ---- drawing (SURVEY.md 8f row f2) --------------------------------------------------------------
  * Paints the people of the last run onto n DEVICE frames uint8 [n, H, W, 3] (contiguous, in place), as the reference's

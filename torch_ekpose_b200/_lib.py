@@ -22,6 +22,7 @@ OVF_PEAKS, OVF_PART, OVF_CANDIDATES, OVF_HUMANS, OVF_BADPEAK = 1, 2, 4, 8, 16
 MAX_PART, MAX_CAND = 256, 2048                                              # EKP_MAX_PART / EKP_MAX_CAND (defaults)
 LIMIT_PEAKS, LIMIT_HUMANS, LIMIT_PART, LIMIT_CAND = 16384, 1024, 1024, 8192  # EKP_LIMIT_*
 DRAW_MAX_SIDE = 16384                                                       # EKP_DRAW_MAX_SIDE
+LIMIT_TRACKS = 512                                                          # EKP_LIMIT_TRACKS
 
 
 class EkpError(RuntimeError):
@@ -86,6 +87,10 @@ SIGNATURES = {
     "ekp_draw_humans": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "ekp_debug_raster_host": (_i, [_i, _i, _i, _i, _i, _i, _i, _vp]),
     "ekp_debug_draw_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _i, _i]),
+    "ekp_track_state_bytes": (C.c_longlong, [_i, _i]),
+    "ekp_track_reset": (_i, [_vp, _vp, _i, _i, _vp]),
+    "ekp_track_humans": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i, _i, _f, _i, _vp, _vp]),
+    "ekp_debug_track_host": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _f, _i, _vp]),
     # the reference operator surface, lib/pafprocess/pafprocess.h:53-59
     "process_paf": (_i, [_i, _i, _i, _vp, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "get_num_humans": (_i, []),

@@ -220,6 +220,7 @@ extern "C" int ekp_create_ex(ekp_ctx** out, int device, int max_batch, int max_h
     if (e == cudaSuccess) e = configure_peaks_sort(max_peaks);
     if (e == cudaSuccess) e = configure_connect(max_part, max_cand);
     if (e == cudaSuccess) e = configure_assemble(max_humans, max_peaks, max_part);
+    if (e == cudaSuccess) e = configure_track();
     if (e != cudaSuccess) { ctx_free(c); return fail(EKP_ERR_CUDA, "context setup: %s", cudaGetErrorString(e)); }
     *out = c;
     return EKP_OK;
@@ -738,6 +739,64 @@ extern "C" int ekp_results_device_peaks(ekp_ctx* c, int n, const ekp_device_peak
         c->launches += 1;
         return (int) EKP_OK;
     });
+}
+
+// ---- tracking (track.cu): reads caller tables, not the context's records, so no after_run ordering --------------------
+extern "C" long long ekp_track_state_bytes(int n_seq, int max_tracks) {
+    if (n_seq < 1 || max_tracks < 1 || max_tracks > EKP_LIMIT_TRACKS) return 0;
+    return (long long) n_seq * (long long) track_seq_bytes(max_tracks);
+}
+
+static int track_state_args(const void* state, int n_seq, int max_tracks, const char* who) {
+    if (!state) return fail(EKP_ERR_ARG, "%s: NULL state", who);
+    if (reinterpret_cast<uintptr_t>(state) & 7u) return fail(EKP_ERR_ARG, "%s: the state is not 8-byte aligned", who);
+    if (n_seq < 1 || max_tracks < 1 || max_tracks > EKP_LIMIT_TRACKS)
+        return fail(EKP_ERR_ARG, "%s: n_seq %d >= 1, max_tracks %d in [1, %d]", who, n_seq, max_tracks, EKP_LIMIT_TRACKS);
+    return EKP_OK;
+}
+
+// the checks ekp_track_humans and ekp_debug_track_host share
+static int track_args(const int* num_humans, const ekp_peak* parts, int n, int max_humans, const void* state, int n_seq,
+                      int max_tracks, float min_oks, int max_age, const int* ids, const char* who) {
+    int rc = track_state_args(state, n_seq, max_tracks, who);
+    if (rc) return rc;
+    if (!num_humans || !parts || !ids) return fail(EKP_ERR_ARG, "%s: NULL table", who);
+    if ((reinterpret_cast<uintptr_t>(num_humans) | reinterpret_cast<uintptr_t>(parts) | reinterpret_cast<uintptr_t>(ids)) & 3u)
+        return fail(EKP_ERR_ARG, "%s: a table is not 4-byte aligned", who);
+    if (n < 1 || n % n_seq) return fail(EKP_ERR_ARG, "%s: %d images are not a multiple of %d sequences", who, n, n_seq);
+    if (max_humans < 1 || max_humans > max_tracks)
+        return fail(EKP_ERR_ARG, "%s: max_humans %d outside [1, max_tracks %d]", who, max_humans, max_tracks);
+    if (max_age < 0) return fail(EKP_ERR_ARG, "%s: max_age %d < 0", who, max_age);
+    if (!(min_oks >= 0.f) || isinf(min_oks)) return fail(EKP_ERR_ARG, "%s: min_oks %g is not a finite non-negative number", who, (double) min_oks);
+    return EKP_OK;
+}
+
+extern "C" int ekp_track_reset(ekp_ctx* c, void* state, int n_seq, int max_tracks, void* stream) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_track_reset: NULL context");
+    int rc = track_state_args(state, n_seq, max_tracks, "ekp_track_reset");
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    CU(cudaMemsetAsync(state, 0, (size_t) ekp_track_state_bytes(n_seq, max_tracks), (cudaStream_t) stream));
+    return EKP_OK;
+}
+
+extern "C" int ekp_track_humans(ekp_ctx* c, const int* num_humans, const ekp_peak* parts, int n, int max_humans, void* state, int n_seq,
+                                int max_tracks, float min_oks, int max_age, int* ids, void* stream) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_track_humans: NULL context");
+    int rc = track_args(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids, "ekp_track_humans");
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    CU(launch_track(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids, (cudaStream_t) stream));
+    c->launches += 1;
+    return EKP_OK;
+}
+
+extern "C" int ekp_debug_track_host(const int* num_humans, const ekp_peak* parts, int n, int max_humans, void* state, int n_seq,
+                                    int max_tracks, float min_oks, int max_age, int* ids) {
+    int rc = track_args(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids, "ekp_debug_track_host");
+    if (rc) return rc;
+    debug_track_host(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids);
+    return EKP_OK;
 }
 
 extern "C" int ekp_set_host_copy(ekp_ctx* c, int enable) {

@@ -46,6 +46,12 @@ cudaError_t launch_results_export(const unsigned char* records, const ResultLayo
                                   const ekp_device_results& out, cudaStream_t stream);
 cudaError_t launch_peaks_export(const unsigned char* records, size_t stride, const ekp_peak* line, const int* part_off, int max_peaks,
                                 int n, const ekp_device_peaks& out, cudaStream_t stream);
+size_t track_seq_bytes(int max_tracks);
+cudaError_t configure_track();
+cudaError_t launch_track(const int* num_humans, const ekp_peak* parts, int n, int max_humans, void* state, int n_seq, int max_tracks,
+                         float min_oks, int max_age, int* ids, cudaStream_t stream);
+void debug_track_host(const int* num_humans, const ekp_peak* parts, int n, int max_humans, void* state, int n_seq, int max_tracks,
+                      float min_oks, int max_age, int* ids);
 void debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask);
 void debug_draw_host(const int* num_humans, const ekp_peak* parts, int max_humans, int map_h, int map_w,
                      unsigned char* frames, int n, int H, int W);

@@ -99,15 +99,20 @@ def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, f
 
 
 def infer_human_tensors(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15,
-                        subset: bool = False, peaks: bool = False):
+                        subset: bool = False, peaks: bool = False, tracker=None):
     """``infer_humans`` with the people left on the GPU: returns (tensors, im_scale), ``tensors`` being the dict of
     CUDA tensors ``PostProcessor.result_tensors(subset=subset)`` returns (per image num_humans, overflow, n_peaks,
     the part table, part and human scores; with ``peaks=True`` also the peak table) and ``im_scale`` that of
     ``get_outputs_batched``.  Nothing waits for the device and nothing raises on a capacity overflow: the caller checks
     ``tensors['overflow']``.  The batch leaves its records on the device (no copy to the host); ``last_postprocessor()``'s
-    host readers still work, at the cost of one download."""
+    host readers still work, at the cost of one download.  With a ``Tracker`` (``tracking.py``) of the same device,
+    ``tensors['track_id']`` (int32 [n, max_humans]) holds each person's id across calls, computed on the export's
+    stream."""
     pafs, heats, im_scale = get_outputs_batched(images, model, preprocess, device)
-    return _postprocess(heats, pafs, frontend, thr, False).result_tensors(subset=subset, peaks=peaks), im_scale
+    tensors = _postprocess(heats, pafs, frontend, thr, False).result_tensors(subset=subset, peaks=peaks)
+    if tracker is not None:
+        tensors["track_id"] = tracker.update(tensors)
+    return tensors, im_scale
 
 
 def infer_and_draw(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15):

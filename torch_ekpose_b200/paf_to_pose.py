@@ -52,6 +52,22 @@ def _dtype16(heat, paf) -> int:
     return 0
 
 
+def _torch_stream(dev, stream):
+    """``stream`` (None: the current stream of ``dev``; a torch stream; or a raw cudaStream_t) as a torch stream, for
+    allocating tensors under the stream that will use them."""
+    if stream is None:
+        return torch.cuda.current_stream(dev)
+    if isinstance(stream, torch.cuda.Stream):
+        return stream
+    return torch.cuda.ExternalStream(int(getattr(stream, "cuda_stream", stream)), device=dev)
+
+
+def _check_out(t, what: str, shape, dt, dev) -> None:
+    """ValueError unless ``t`` is a contiguous ``dt`` tensor of ``shape`` on ``dev`` (the ``out=`` buffers)."""
+    if not (_is_tensor(t) and t.device == dev and t.dtype == dt and tuple(t.shape) == tuple(shape) and t.is_contiguous()):
+        raise ValueError(f"{what} must be a contiguous {dt} tensor {list(shape)} on {dev}")
+
+
 class PostProcessor:
     """A libekpose_b200 context: stages 1-5 for batches of up to ``max_batch`` images.
 
@@ -261,20 +277,12 @@ class PostProcessor:
         dev = torch.device("cuda", self.device)
         specs = self._result_specs(n, subset, peaks)
         if out is None:
-            if stream is None:
-                st = torch.cuda.current_stream(dev)
-            elif isinstance(stream, torch.cuda.Stream):
-                st = stream
-            else:
-                st = torch.cuda.ExternalStream(int(getattr(stream, "cuda_stream", stream)), device=dev)
-            with torch.cuda.device(dev), torch.cuda.stream(st):
+            stream = _torch_stream(dev, stream)
+            with torch.cuda.device(dev), torch.cuda.stream(stream):
                 out = {name: torch.empty(shape, dtype=dt, device=dev) for name, shape, dt in specs}
-            stream = st
         else:
             for name, shape, dt in specs:
-                t = out.get(name) if isinstance(out, dict) else None
-                if not (_is_tensor(t) and t.device == dev and t.dtype == dt and tuple(t.shape) == shape and t.is_contiguous()):
-                    raise ValueError(f"out[{name!r}] must be a contiguous {dt} tensor {list(shape)} on {dev}")
+                _check_out(out.get(name) if isinstance(out, dict) else None, f"out[{name!r}]", shape, dt, dev)
         tabs = _lib.DeviceResults(*(out[k].data_ptr() if k in out and (k != "subset" or subset) else None
                                     for k in ("num_humans", "overflow", "n_peaks", "subset", "parts", "scores")))
         st = self._stream(stream)
