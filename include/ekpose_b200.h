@@ -264,6 +264,84 @@ int ekp_track_humans(ekp_ctx *ctx, const int *num_humans, const ekp_peak *parts,
 int ekp_debug_track_host(const int *num_humans, const ekp_peak *parts, int n, int max_humans, void *state, int n_seq,
                          int max_tracks, float min_oks, int max_age, int *ids);
 
+/* ---- COCO keypoint evaluation: pycocotools' COCOeval(iouType='keypoints') on the device ------------------------------
+ * Scores detected people against COCO person-keypoint ground truth, one category, and writes accumulate()'s precision,
+ * recall and scores arrays, equal bit for bit to pycocotools' (float64 throughout).  Inputs are padded per-image tables
+ * of n_img images: image order is row order (the Python packers sort by image id, as pycocotools' np.unique does), and
+ * within an image rows are in annotation order (gt) or result-list order (dt); counts are clamped to [0, max_gt] /
+ * [0, max_dt].  The rules, as pycocotools states them:
+ *   dt area      (loadRes) over all 17 keypoints, absent (0, 0, 0) triples included: (max x - min x) * (max y - min y).
+ *   gt ignore    (_prepare) iscrowd or num_keypoints == 0, packed into `ignore` by the caller.
+ *   dt order     a stable sort by descending score, truncated to max_det; -0.0 and +0.0 compare equal.
+ *   OKS          (computeOks) vars = (2 sigma)^2 with pycocotools' sigmas; k1 = gt keypoints with v > 0.  k1 > 0:
+ *                dx = xd - xg over those keypoints; k1 == 0: dx = max(0, x0 - xd) + max(0, xd - x1) with x0 = bx - bw,
+ *                x1 = bx + 2 bw from the gt bbox (likewise y), over all 17.  e = (dx^2 + dy^2) / vars / (area + 2^-52) / 2,
+ *                oks = sum(exp(-e)) / len(e), the sum in numpy's pairwise order (sequential below 8 terms, else eight
+ *                accumulators over the multiple-of-8 prefix, ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), then the rest).
+ *   matching     (evaluateImg) per image, area range a = [lo, hi] and threshold t: gts stable-sorted by
+ *                _ignore = ignore or area outside [lo, hi]; each dt in order starts from iou = min(t, 1 - 1e-10) and
+ *                scans the gts, skipping one already matched at t unless it is a crowd, stopping at the first ignored gt
+ *                once its match is a non-ignored one, skipping oks < iou, else taking iou = oks and that gt (so among equal
+ *                OKS the last gt wins).  A matched dt is ignored when its gt is; an unmatched one when its own area is
+ *                outside [lo, hi].
+ *   accumulate   all kept dts of all images, concatenated in image order and stable-sorted by descending score;
+ *                npig = non-ignored gts of area a (0: that area's entries stay -1); tp / fp running counts in float64,
+ *                rc = tp / npig, pr = tp / ((fp + tp) + 2^-52), pr replaced by its running maximum from the end;
+ *                i = searchsorted(rc, recThrs[r], 'left'), precision = pr[i] and scores = the i-th sorted score, both 0
+ *                when i is past the end; recall = rc[-1], or 0 with no detections.
+ * The thresholds are inputs: iou_thrs [T], rec_thrs [R] and area_rng [A][2] (pycocotools' np.linspace values and
+ * [[0, 1e10], [32^2, 96^2], [96^2, 1e10]] for its keypoint defaults).  Non-finite inputs give unspecified numbers, never
+ * an out-of-bounds access.  Every pointer is a caller-owned DEVICE pointer (host pointers for the test hook), 8-byte
+ * aligned; the tables are float64 where pycocotools keeps floats, int32 otherwise. */
+typedef struct ekp_coco_gt {
+    const int *count;          /* [n_img]                  ground-truth people per image */
+    const double *keypoints;   /* [n_img, max_gt, 17, 3]   (x, y, v) in COCO keypoint order */
+    const double *bbox;        /* [n_img, max_gt, 4]       (x, y, w, h) */
+    const double *area;        /* [n_img, max_gt] */
+    const int *iscrowd;        /* [n_img, max_gt] */
+    const int *ignore;         /* [n_img, max_gt]          iscrowd || num_keypoints == 0 */
+} ekp_coco_gt;
+typedef struct ekp_coco_dt {
+    const int *count;          /* [n_img]                  detections per image */
+    const double *keypoints;   /* [n_img, max_dt, 17, 3] */
+    const double *score;       /* [n_img, max_dt] */
+} ekp_coco_dt;
+typedef struct ekp_coco_eval_out {
+    double *precision;         /* [T, R, A]   accumulate()'s precision[:, :, 0, :, 0] */
+    double *recall;            /* [T, A]      recall[:, 0, :, 0] */
+    double *scores;            /* [T, R, A]   scores[:, :, 0, :, 0] */
+    /* optional (NULL: not written), for tests; dt index d = the rank in the image's score order */
+    int *dt_match;             /* [n_img, A, T, max_det]   the matched gt row, or -1 (also for d past the kept dts) */
+    int *dt_ignore;            /* [n_img, A, T, max_det]   evaluateImg's dtIgnore (0 past the kept dts) */
+    double *oks;               /* [n_img, max_det, max_gt] computeOks' matrix, gts in row order (0 past the counts) */
+} ekp_coco_eval_out;
+/* Limits.  The per-image OKS matrix (max_det x max_gt float64) lives in the shared memory of the image's block, beside
+ * the image's sort keys (max_dt) and one matched flag per walk and gt: at the limits 116.7 of the 227 KB a block has. */
+#define EKP_COCO_LIMIT_CURVES 32       /* T * A: one tp and one fp bit per curve and detection */
+#define EKP_COCO_LIMIT_REC 1024        /* R */
+#define EKP_COCO_LIMIT_GT 128          /* max_gt */
+#define EKP_COCO_LIMIT_DT 1024         /* max_dt */
+#define EKP_COCO_LIMIT_DET 100         /* max_det */
+#define EKP_COCO_LIMIT_IMAGES 1048576  /* n_img */
+/* Bytes of the workspace of one evaluation (256-byte aligned); 0 when a size is outside its limit.  It grows with
+ * n_img x max_det (about 51 bytes a slot), and does not depend on max_gt, max_dt or n_iou. */
+long long ekp_coco_eval_workspace_bytes(int n_img, int max_gt, int max_dt, int max_det, int n_area, int n_iou);
+/* One evaluation, asynchronous on `stream`: 29 kernel launches (one block per image, eight 8-bit passes of a radix sort
+ * of n_img x max_det slots, four accumulate steps), counted in ekp_kernel_launches; no host wait, no allocation.  Every
+ * output entry is written.  The workspace is the caller's (at least ekp_coco_eval_workspace_bytes), may be reused by
+ * calls ordered after this one, must be 256-byte aligned, and is not read before it is written.  The context supplies the device, the error
+ * reporting and the launch count.  EKP_ERR_ARG for a NULL context, table or required output, a size outside its limit
+ * (n_img, max_gt, max_dt, max_det, T, R, A >= 1; T * A <= EKP_COCO_LIMIT_CURVES) or a pointer that is not 8-byte
+ * aligned. */
+int ekp_coco_eval_kpts(ekp_ctx *ctx, const ekp_coco_gt *gt, int max_gt, const ekp_coco_dt *dt, int max_dt, int n_img,
+                       int max_det, const double *iou_thrs, int T, const double *rec_thrs, int R, const double *area_rng,
+                       int A, void *workspace, const ekp_coco_eval_out *out, void *stream);
+/* Test hook for ekp_coco_eval_kpts: the same per-image and accumulate code run serially on the CPU on HOST buffers (the
+ * radix sort replaced by std::stable_sort on the same keys), with the same checks.  It is not a CPU path. */
+int ekp_debug_coco_eval_host(const ekp_coco_gt *gt, int max_gt, const ekp_coco_dt *dt, int max_dt, int n_img, int max_det,
+                             const double *iou_thrs, int T, const double *rec_thrs, int R, const double *area_rng, int A,
+                             const ekp_coco_eval_out *out);
+
 /* ---- drawing (SURVEY.md 8f row f2) --------------------------------------------------------------
  * Paints the people of the last run onto n DEVICE frames uint8 [n, H, W, 3] (contiguous, in place), as the reference's
  * draw_humans (lib/utils/common.py:252-275) paints each image's list[Human]: byte for byte.  Per human of the table, in

@@ -23,6 +23,7 @@ MAX_PART, MAX_CAND = 256, 2048                                              # EK
 LIMIT_PEAKS, LIMIT_HUMANS, LIMIT_PART, LIMIT_CAND = 16384, 1024, 1024, 8192  # EKP_LIMIT_*
 DRAW_MAX_SIDE = 16384                                                       # EKP_DRAW_MAX_SIDE
 LIMIT_TRACKS = 512                                                          # EKP_LIMIT_TRACKS
+COCO_LIMIT_CURVES, COCO_LIMIT_REC, COCO_LIMIT_GT, COCO_LIMIT_DT, COCO_LIMIT_DET, COCO_LIMIT_IMAGES = 32, 1024, 128, 1024, 100, 1 << 20
 
 
 class EkpError(RuntimeError):
@@ -46,6 +47,20 @@ class DeviceResults(C.Structure):  # ekp_device_results: device pointers, None =
 
 class DevicePeaks(C.Structure):  # ekp_device_peaks: device pointers, None = that table is not written
     _fields_ = [("n_peaks", C.c_void_p), ("peaks", C.c_void_p), ("part_off", C.c_void_p)]
+
+
+class CocoGt(C.Structure):  # ekp_coco_gt: device pointers (host pointers for the test hook)
+    _fields_ = [("count", C.c_void_p), ("keypoints", C.c_void_p), ("bbox", C.c_void_p), ("area", C.c_void_p),
+                ("iscrowd", C.c_void_p), ("ignore", C.c_void_p)]
+
+
+class CocoDt(C.Structure):  # ekp_coco_dt
+    _fields_ = [("count", C.c_void_p), ("keypoints", C.c_void_p), ("score", C.c_void_p)]
+
+
+class CocoEvalOut(C.Structure):  # ekp_coco_eval_out: None = that optional output is not written
+    _fields_ = [("precision", C.c_void_p), ("recall", C.c_void_p), ("scores", C.c_void_p), ("dt_match", C.c_void_p),
+                ("dt_ignore", C.c_void_p), ("oks", C.c_void_p)]
 
 
 # every symbol include/ekpose_b200.h declares: (restype, argtypes)
@@ -91,6 +106,11 @@ SIGNATURES = {
     "ekp_track_reset": (_i, [_vp, _vp, _i, _i, _vp]),
     "ekp_track_humans": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i, _i, _f, _i, _vp, _vp]),
     "ekp_debug_track_host": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _f, _i, _vp]),
+    "ekp_coco_eval_workspace_bytes": (C.c_longlong, [_i, _i, _i, _i, _i, _i]),
+    "ekp_coco_eval_kpts": (_i, [_vp, C.POINTER(CocoGt), _i, C.POINTER(CocoDt), _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp,
+                                C.POINTER(CocoEvalOut), _vp]),
+    "ekp_debug_coco_eval_host": (_i, [C.POINTER(CocoGt), _i, C.POINTER(CocoDt), _i, _i, _i, _vp, _i, _vp, _i, _vp, _i,
+                                      C.POINTER(CocoEvalOut)]),
     # the reference operator surface, lib/pafprocess/pafprocess.h:53-59
     "process_paf": (_i, [_i, _i, _i, _vp, _i, _i, _i, _vp, _i, _i, _i, _vp]),
     "get_num_humans": (_i, []),

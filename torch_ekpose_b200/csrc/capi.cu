@@ -221,6 +221,7 @@ extern "C" int ekp_create_ex(ekp_ctx** out, int device, int max_batch, int max_h
     if (e == cudaSuccess) e = configure_connect(max_part, max_cand);
     if (e == cudaSuccess) e = configure_assemble(max_humans, max_peaks, max_part);
     if (e == cudaSuccess) e = configure_track();
+    if (e == cudaSuccess) e = configure_coco_eval();
     if (e != cudaSuccess) { ctx_free(c); return fail(EKP_ERR_CUDA, "context setup: %s", cudaGetErrorString(e)); }
     *out = c;
     return EKP_OK;
@@ -796,6 +797,62 @@ extern "C" int ekp_debug_track_host(const int* num_humans, const ekp_peak* parts
     int rc = track_args(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids, "ekp_debug_track_host");
     if (rc) return rc;
     debug_track_host(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids);
+    return EKP_OK;
+}
+
+// ---- COCO keypoint evaluation (coco_eval.cu): caller tables and workspace, no after_run ordering ---------------------
+static bool coco_sizes_ok(int n_img, int max_gt, int max_dt, int max_det, int A, int T) {
+    return n_img >= 1 && n_img <= EKP_COCO_LIMIT_IMAGES && max_gt >= 1 && max_gt <= EKP_COCO_LIMIT_GT && max_dt >= 1 &&
+           max_dt <= EKP_COCO_LIMIT_DT && max_det >= 1 && max_det <= EKP_COCO_LIMIT_DET && A >= 1 && T >= 1 &&
+           A * T <= EKP_COCO_LIMIT_CURVES;
+}
+
+extern "C" long long ekp_coco_eval_workspace_bytes(int n_img, int max_gt, int max_dt, int max_det, int n_area, int n_iou) {
+    if (!coco_sizes_ok(n_img, max_gt, max_dt, max_det, n_area, n_iou)) return 0;
+    return (long long) coco_eval_ws_bytes(n_img, max_det, n_area);
+}
+
+// the checks ekp_coco_eval_kpts and ekp_debug_coco_eval_host share
+static int coco_args_ok(const ekp_coco_gt* gt, int max_gt, const ekp_coco_dt* dt, int max_dt, int n_img, int max_det,
+                        const double* iou, int T, const double* rec, int R, const double* area, int A, const ekp_coco_eval_out* out,
+                        const char* who) {
+    if (!gt || !dt || !out) return fail(EKP_ERR_ARG, "%s: NULL %s", who, !gt ? "gt" : !dt ? "dt" : "out");
+    if (!coco_sizes_ok(n_img, max_gt, max_dt, max_det, A, T) || R < 1 || R > EKP_COCO_LIMIT_REC)
+        return fail(EKP_ERR_ARG, "%s: n_img %d, max_gt %d, max_dt %d, max_det %d, T %d, R %d, A %d outside the limits", who,
+                    n_img, max_gt, max_dt, max_det, T, R, A);
+    const void* need[] = {gt->count, gt->keypoints, gt->bbox, gt->area, gt->iscrowd, gt->ignore, dt->count, dt->keypoints,
+                          dt->score, iou, rec, area, out->precision, out->recall, out->scores};
+    for (const void* p : need) {
+        if (!p) return fail(EKP_ERR_ARG, "%s: NULL table, threshold or output", who);
+        if (reinterpret_cast<uintptr_t>(p) & 7u) return fail(EKP_ERR_ARG, "%s: a pointer is not 8-byte aligned", who);
+    }
+    const void* opt[] = {out->dt_match, out->dt_ignore, out->oks};
+    for (const void* p : opt)
+        if (reinterpret_cast<uintptr_t>(p) & 7u) return fail(EKP_ERR_ARG, "%s: an optional output is not 8-byte aligned", who);
+    return EKP_OK;
+}
+
+extern "C" int ekp_coco_eval_kpts(ekp_ctx* c, const ekp_coco_gt* gt, int max_gt, const ekp_coco_dt* dt, int max_dt, int n_img,
+                                  int max_det, const double* iou_thrs, int T, const double* rec_thrs, int R, const double* area_rng,
+                                  int A, void* workspace, const ekp_coco_eval_out* out, void* stream) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_coco_eval_kpts: NULL context");
+    int rc = coco_args_ok(gt, max_gt, dt, max_dt, n_img, max_det, iou_thrs, T, rec_thrs, R, area_rng, A, out, "ekp_coco_eval_kpts");
+    if (rc) return rc;
+    if (!workspace || reinterpret_cast<uintptr_t>(workspace) & 255u)
+        return fail(EKP_ERR_ARG, "ekp_coco_eval_kpts: the workspace is NULL or not 256-byte aligned");
+    CU(cudaSetDevice(c->device));
+    CU(launch_coco_eval(*gt, max_gt, *dt, max_dt, n_img, max_det, iou_thrs, T, rec_thrs, R, area_rng, A, workspace, *out,
+                        (cudaStream_t) stream));
+    c->launches += coco_eval_launches();
+    return EKP_OK;
+}
+
+extern "C" int ekp_debug_coco_eval_host(const ekp_coco_gt* gt, int max_gt, const ekp_coco_dt* dt, int max_dt, int n_img, int max_det,
+                                        const double* iou_thrs, int T, const double* rec_thrs, int R, const double* area_rng, int A,
+                                        const ekp_coco_eval_out* out) {
+    int rc = coco_args_ok(gt, max_gt, dt, max_dt, n_img, max_det, iou_thrs, T, rec_thrs, R, area_rng, A, out, "ekp_debug_coco_eval_host");
+    if (rc) return rc;
+    debug_coco_eval_host(*gt, max_gt, *dt, max_dt, n_img, max_det, iou_thrs, T, rec_thrs, R, area_rng, A, *out);
     return EKP_OK;
 }
 

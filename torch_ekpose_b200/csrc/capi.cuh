@@ -52,6 +52,16 @@ cudaError_t launch_track(const int* num_humans, const ekp_peak* parts, int n, in
                          float min_oks, int max_age, int* ids, cudaStream_t stream);
 void debug_track_host(const int* num_humans, const ekp_peak* parts, int n, int max_humans, void* state, int n_seq, int max_tracks,
                       float min_oks, int max_age, int* ids);
+cudaError_t configure_coco_eval();
+size_t coco_eval_ws_bytes(long long n_img, long long max_det, int A);
+size_t coco_img_smem_bytes(int max_gt, int max_dt, int max_det);
+int coco_eval_launches();
+cudaError_t launch_coco_eval(const ekp_coco_gt& gt, int max_gt, const ekp_coco_dt& dt, int max_dt, int n_img, int max_det,
+                             const double* iou, int T, const double* rec, int R, const double* area, int A, void* ws,
+                             const ekp_coco_eval_out& out, cudaStream_t st);
+void debug_coco_eval_host(const ekp_coco_gt& gt, int max_gt, const ekp_coco_dt& dt, int max_dt, int n_img, int max_det,
+                          const double* iou, int T, const double* rec, int R, const double* area, int A,
+                          const ekp_coco_eval_out& out);
 void debug_raster_host(int kind, int x0, int y0, int x1, int y1, int H, int W, unsigned char* mask);
 void debug_draw_host(const int* num_humans, const ekp_peak* parts, int max_humans, int map_h, int map_w,
                      unsigned char* frames, int n, int H, int W);

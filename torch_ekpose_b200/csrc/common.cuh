@@ -123,6 +123,16 @@ inline cudaError_t raise_dynamic_smem_limit(Kernel kernel, size_t bytes) {
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bytes);
 }
 
+// pycocotools' keypoint variances: sigmas = array([...]) / 10.0, vars = (sigmas * 2) ** 2, in float64 (on the host,
+// into the kernels' arguments).  One copy for the tracker's similarity (track.cu) and the COCO evaluation (coco_eval.cu).
+inline void oks_vars(double var[17]) {
+    const double s[17] = {.26, .25, .25, .35, .35, .79, .79, .72, .72, .62, .62, 1.07, 1.07, .87, .87, .89, .89};
+    for (int j = 0; j < 17; j++) {
+        const double sg = s[j] / 10.0;
+        var[j] = (sg * 2) * (sg * 2);
+    }
+}
+
 // launch parameter blocks --------------------------------------------------------------------
 struct AsmParams {
     const ekp_peak* line;      // [n][max_peaks] part-sorted peak table

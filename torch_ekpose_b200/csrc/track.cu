@@ -96,16 +96,6 @@ HD int coco_part(int j) {
 #endif
 }
 
-// pycocotools' variances: sigmas = array([...]) / 10.0, vars = (sigmas * 2) ** 2, in float64 (on the host, into the
-// kernel's arguments)
-static void oks_vars(double* var) {
-    const double s[kCoco] = {.26, .25, .25, .35, .35, .79, .79, .72, .72, .62, .62, 1.07, 1.07, .87, .87, .89, .89};
-    for (int j = 0; j < kCoco; j++) {
-        const double sg = s[j] / 10.0;
-        var[j] = (sg * 2) * (sg * 2);
-    }
-}
-
 // the COCO pose of one row of a part table (ekp_peak [18]: id -1 = absent)
 HD void load_pose(const ekp_peak* row, PersonPose& out) {
     unsigned mask = 0;

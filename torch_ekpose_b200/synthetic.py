@@ -29,17 +29,21 @@ _TPL = np.array([(.50, .08), (.50, .20), (.35, .20), (.30, .38), (.28, .55), (.6
 SHAPES = {"368x432": (46, 54), "656x368": (46, 82), "1312x736": (92, 164)}
 
 
-def make_scene(h: int, w: int, people: int, seed: int, noise: bool = True):
-    """One image: returns (heat[h,w,19], paf[h,w,38]) float32, HWC like estimator.get_outputs."""
+def make_scene(h: int, w: int, people: int, seed: int, noise: bool = True, return_truth: bool = False):
+    """One image: returns (heat[h,w,19], paf[h,w,38]) float32, HWC like estimator.get_outputs.  return_truth=True adds
+    a third item, truth float64 [people, 18, 2]: every person's 18 joints (x, y) in reference part order, in the
+    stride-8 map's pixels (the centres of the heat blobs)."""
     rng = np.random.default_rng(seed)
     yy, xx = np.mgrid[0:h, 0:w].astype(np.float64)
     heat = np.zeros((h, w, 19), np.float64)
     paf = np.zeros((h, w, 38), np.float64)
-    for _ in range(people):
+    truth = np.zeros((people, 18, 2), np.float64)
+    for person in range(people):
         s = rng.uniform(0.35, 0.7) * h
         cx = rng.uniform(0.1, 0.9) * w
         cy = rng.uniform(0.05, 0.4) * h
         kp = _TPL * np.array([0.6 * s, s]) + np.array([cx - 0.3 * s, cy]) + rng.normal(0, 0.3, (18, 2))
+        truth[person] = kp
         amp = rng.uniform(0.6, 1.0, 18)
         for k in range(18):
             d2 = (xx - kp[k, 0]) ** 2 + (yy - kp[k, 1]) ** 2
@@ -61,22 +65,26 @@ def make_scene(h: int, w: int, people: int, seed: int, noise: bool = True):
         heat[:, :, :18] += rng.normal(0, 0.005, (h, w, 18))
         paf += rng.normal(0, 0.01, (h, w, 38))
     heat[:, :, 18] = np.maximum(1 - heat[:, :, :18].max(axis=2), 0)
+    if return_truth:
+        return heat.astype(np.float32), paf.astype(np.float32), truth
     return heat.astype(np.float32), paf.astype(np.float32)
 
 
-def make_batch(batch: int, h: int, w: int, people_range=(1, 6), seed: int = 0, layout: str = "nchw"):
+def make_batch(batch: int, h: int, w: int, people_range=(1, 6), seed: int = 0, layout: str = "nchw",
+               return_truth: bool = False):
     """A batch of scenes.  layout 'nchw' (what the network emits, vgg2016.py:105) or 'nhwc'.
 
     Scene i uses seed `1000*seed + i` and people count cycling through people_range inclusive.
-    Returns (heat, paf) float32 arrays.
+    Returns (heat, paf) float32 arrays; return_truth=True adds the list of the scenes' truth arrays (make_scene).
     """
     lo, hi = people_range
-    heats, pafs = [], []
+    heats, pafs, truths = [], [], []
     for i in range(batch):
         p = lo + (i % (hi - lo + 1))
-        hm, pf = make_scene(h, w, p, 1000 * seed + i)
-        heats.append(hm)
-        pafs.append(pf)
+        scene = make_scene(h, w, p, 1000 * seed + i, return_truth=return_truth)
+        heats.append(scene[0])
+        pafs.append(scene[1])
+        truths.append(scene[2] if return_truth else None)
     heat = np.stack(heats)
     paf = np.stack(pafs)
     if layout == "nchw":
@@ -84,4 +92,6 @@ def make_batch(batch: int, h: int, w: int, people_range=(1, 6), seed: int = 0, l
         paf = np.ascontiguousarray(paf.transpose(0, 3, 1, 2))
     elif layout != "nhwc":
         raise ValueError("layout must be 'nchw' or 'nhwc'")
+    if return_truth:
+        return heat, paf, truths
     return heat, paf
