@@ -21,7 +21,8 @@
  *    (ekp_results, ekp_results_humans: these wait for the run) or into caller-owned device buffers, ordered on a
  *    stream with no host wait (ekp_results_device, ekp_results_device_peaks).  A caller that reads them only on the
  *    device can also skip each batch's copy of the result records to the host (ekp_set_host_copy), and give its people
- *    stable ids across video frames on the device (ekp_track_humans).
+ *    stable ids across video frames on the device (ekp_track_humans), and smooth their keypoints per id
+ *    (ekp_smooth_humans).
  *
  * All functions return EKP_OK (0) or a negative ekp_status; ekp_last_error() returns a
  * thread-local human-readable message for the last failure.  Nothing aborts.
@@ -263,6 +264,59 @@ int ekp_track_humans(ekp_ctx *ctx, const int *num_humans, const ekp_peak *parts,
  * arguments and checks.  It is not a CPU path of the tracker. */
 int ekp_debug_track_host(const int *num_humans, const ekp_peak *parts, int n, int max_humans, void *state, int n_seq,
                          int max_tracks, float min_oks, int max_age, int *ids);
+
+/* ---- smoothing: One Euro filtered keypoints across video frames, per track --------------------------------------------
+ * Smooths the people's keypoints from frame to frame with a One Euro filter (Casiez, Roussel, Vogel, CHI 2012) per track
+ * id, part and axis, on the device human tables (ekp_results_device's num_humans and parts) and the ids ekp_track_humans
+ * wrote for them.  Both front-ends report integer map pixels, so a still person's keypoints jump by a pixel or more
+ * between frames; the filter removes that jitter at low speed and follows fast motion with little lag.
+ * A call takes n images and n_seq sequences as ekp_track_humans does (n % n_seq == 0, F = n / n_seq, image i is frame
+ * i % F of sequence i / F).  Each sequence keeps its own frame counter and up to max_tracks entries, one per track id,
+ * in `state`, across calls.  An entry holds, per reference part (all 18, the neck included, in part order) and axis, the
+ * filter values xh, dxh and the frame of the part's last sample.  For row p < min(num_humans[i], max_humans) with
+ * id = ids[i][p]:
+ *   id < 0      the row is passed through: its output is its raw coordinates, and it touches no entry.
+ *   lookup      the row uses the entry of its id.  Without one, it opens one: in a free entry if there is one, else in
+ *               the entry with the smallest (last_seen, id) among those not seen in this frame.  A frame first resolves
+ *               every row whose id already has an entry, and only then opens entries, in row order: a birth never
+ *               evicts an entry a later row of the same frame uses.
+ *   expiry      an entry last seen at frame f0 is dropped at frame f0 + max_age + 2 (the tracker's rule).
+ *   duplicates  ids within a frame must be distinct; duplicates give unspecified coordinates, never an out-of-bounds
+ *               access.
+ * With the (n_seq, max_tracks, max_age) of the ekp_track_humans call that produced the ids, the live entries are exactly
+ * the tracker's live tracks, so a filter restarts only when its track is born.
+ * Per present part (parts[..].id >= 0) and axis, with the raw value x = (double) coordinate at frame f, a part's first
+ * sample in its entry (an opened entry has none) sets xh = x, dxh = 0; every later one, with g = f - (frame of the
+ * part's last sample) and pi the double nearest pi, does in this order, each an IEEE float64 operation, uncontracted:
+ *     te = (double) g / fps            tau_d = 1.0 / ((2.0 * pi) * d_cutoff)     a_d = 1.0 / (1.0 + tau_d / te)
+ *     dx = (x - xh) / te               dxh = a_d * dx + (1.0 - a_d) * dxh
+ *     c = min_cutoff + beta * fabs(dxh)
+ *     tau = 1.0 / ((2.0 * pi) * c)     a = 1.0 / (1.0 + tau / te)                xh = a * x + (1.0 - a) * xh
+ * An absent part leaves its values as they are: its next sample uses the real gap g.
+ * xy float32 [n, max_humans, 18, 2] gets (float) xh, rounded to nearest, for every present part of a row with an entry,
+ * the raw coordinates for the present parts of passed-through rows, and 0.0f for absent parts and rows from num_humans[i]
+ * on, so a dirty buffer is fully overwritten; presence stays readable from parts[..., 3].  Coordinates are map pixels
+ * like the tables' (frame rates, cutoffs and beta are per frame of fps and per pixel accordingly).
+ * Every pointer is a caller-owned DEVICE pointer: the tables, ids and xy 4-byte aligned, the state 8-byte aligned.  The
+ * state's layout is private; its size depends only on (n_seq, max_tracks), so it outlives any context.  Frame counters
+ * are 32-bit.  ekp_smooth_humans is one kernel launch (one block per sequence, counted in ekp_kernel_launches),
+ * asynchronous on `stream`; it never waits on the host and never allocates.  The context only supplies the device and
+ * the error reporting.  EKP_ERR_ARG for a NULL pointer, n < 1 or n % n_seq != 0, max_humans outside [1, max_tracks],
+ * max_tracks outside [1, EKP_LIMIT_TRACKS], max_age < 0, an fps, min_cutoff or d_cutoff that is not finite and
+ * positive, a beta that is not finite and non-negative, or a misaligned pointer. */
+/* Bytes of a state for n_seq sequences of up to max_tracks entries (16 per sequence and 728 per entry); 0 when n_seq < 1 or max_tracks is
+ * outside [1, EKP_LIMIT_TRACKS]. */
+long long ekp_smooth_state_bytes(int n_seq, int max_tracks);
+/* Clears a state asynchronously on `stream` (cudaMemsetAsync): no entries, frame 0 in every sequence. */
+int ekp_smooth_reset(ekp_ctx *ctx, void *state, int n_seq, int max_tracks, void *stream);
+int ekp_smooth_humans(ekp_ctx *ctx, const int *num_humans, const ekp_peak *parts, const int *ids, int n, int max_humans,
+                      void *state, int n_seq, int max_tracks, int max_age, double fps, double min_cutoff, double beta,
+                      double d_cutoff, float *xy, void *stream);
+/* Test hook for ekp_smooth_humans: the same code, run serially on the CPU on HOST buffers (and a host state), with the
+ * same arguments and checks.  It is not a CPU path of the smoother. */
+int ekp_debug_smooth_host(const int *num_humans, const ekp_peak *parts, const int *ids, int n, int max_humans, void *state,
+                          int n_seq, int max_tracks, int max_age, double fps, double min_cutoff, double beta, double d_cutoff,
+                          float *xy);
 
 /* ---- COCO keypoint evaluation: pycocotools' COCOeval(iouType='keypoints') on the device ------------------------------
  * Scores detected people against COCO person-keypoint ground truth, one category, and writes accumulate()'s precision,

@@ -64,7 +64,7 @@ class CocoEvalOut(C.Structure):  # ekp_coco_eval_out: None = that optional outpu
 
 
 # every symbol include/ekpose_b200.h declares: (restype, argtypes)
-_vp, _i, _f = C.c_void_p, C.c_int, C.c_float
+_vp, _i, _f, _d = C.c_void_p, C.c_int, C.c_float, C.c_double
 SIGNATURES = {
     "ekp_create": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _i, _i]),
     "ekp_create_ex": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _i, _i, _i, _i]),
@@ -106,6 +106,10 @@ SIGNATURES = {
     "ekp_track_reset": (_i, [_vp, _vp, _i, _i, _vp]),
     "ekp_track_humans": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i, _i, _f, _i, _vp, _vp]),
     "ekp_debug_track_host": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _f, _i, _vp]),
+    "ekp_smooth_state_bytes": (C.c_longlong, [_i, _i]),
+    "ekp_smooth_reset": (_i, [_vp, _vp, _i, _i, _vp]),
+    "ekp_smooth_humans": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp, _i, _i, _i, _d, _d, _d, _d, _vp, _vp]),
+    "ekp_debug_smooth_host": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i, _i, _i, _d, _d, _d, _d, _vp]),
     "ekp_coco_eval_workspace_bytes": (C.c_longlong, [_i, _i, _i, _i, _i, _i]),
     "ekp_coco_eval_kpts": (_i, [_vp, C.POINTER(CocoGt), _i, C.POINTER(CocoDt), _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp,
                                 C.POINTER(CocoEvalOut), _vp]),

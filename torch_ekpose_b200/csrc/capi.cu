@@ -221,6 +221,7 @@ extern "C" int ekp_create_ex(ekp_ctx** out, int device, int max_batch, int max_h
     if (e == cudaSuccess) e = configure_connect(max_part, max_cand);
     if (e == cudaSuccess) e = configure_assemble(max_humans, max_peaks, max_part);
     if (e == cudaSuccess) e = configure_track();
+    if (e == cudaSuccess) e = configure_smooth();
     if (e == cudaSuccess) e = configure_coco_eval();
     if (e != cudaSuccess) { ctx_free(c); return fail(EKP_ERR_CUDA, "context setup: %s", cudaGetErrorString(e)); }
     *out = c;
@@ -797,6 +798,66 @@ extern "C" int ekp_debug_track_host(const int* num_humans, const ekp_peak* parts
     int rc = track_args(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids, "ekp_debug_track_host");
     if (rc) return rc;
     debug_track_host(num_humans, parts, n, max_humans, state, n_seq, max_tracks, min_oks, max_age, ids);
+    return EKP_OK;
+}
+
+// ---- smoothing (smooth.cu): reads caller tables and ids, like the tracker ------------------------------------------------
+extern "C" long long ekp_smooth_state_bytes(int n_seq, int max_tracks) {
+    if (n_seq < 1 || max_tracks < 1 || max_tracks > EKP_LIMIT_TRACKS) return 0;
+    return (long long) n_seq * (long long) smooth_state_seq_bytes(max_tracks);
+}
+
+// the checks ekp_smooth_humans and ekp_debug_smooth_host share
+static int smooth_args_ok(const int* num_humans, const ekp_peak* parts, const int* ids, int n, int max_humans, const void* state,
+                          int n_seq, int max_tracks, int max_age, double fps, double min_cutoff, double beta, double d_cutoff,
+                          const float* xy, const char* who) {
+    int rc = track_state_args(state, n_seq, max_tracks, who);
+    if (rc) return rc;
+    if (!num_humans || !parts || !ids || !xy) return fail(EKP_ERR_ARG, "%s: NULL table", who);
+    if ((reinterpret_cast<uintptr_t>(num_humans) | reinterpret_cast<uintptr_t>(parts) | reinterpret_cast<uintptr_t>(ids) |
+         reinterpret_cast<uintptr_t>(xy)) & 3u)
+        return fail(EKP_ERR_ARG, "%s: a table is not 4-byte aligned", who);
+    if (n < 1 || n % n_seq) return fail(EKP_ERR_ARG, "%s: %d images are not a multiple of %d sequences", who, n, n_seq);
+    if (max_humans < 1 || max_humans > max_tracks)
+        return fail(EKP_ERR_ARG, "%s: max_humans %d outside [1, max_tracks %d]", who, max_humans, max_tracks);
+    if (max_age < 0) return fail(EKP_ERR_ARG, "%s: max_age %d < 0", who, max_age);
+    const double pos[3] = {fps, min_cutoff, d_cutoff};
+    for (double v : pos)
+        if (!(v > 0.0) || isinf(v)) return fail(EKP_ERR_ARG, "%s: fps %g, min_cutoff %g, d_cutoff %g must be finite and positive", who, fps, min_cutoff, d_cutoff);
+    if (!(beta >= 0.0) || isinf(beta)) return fail(EKP_ERR_ARG, "%s: beta %g is not a finite non-negative number", who, beta);
+    return EKP_OK;
+}
+
+extern "C" int ekp_smooth_reset(ekp_ctx* c, void* state, int n_seq, int max_tracks, void* stream) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_smooth_reset: NULL context");
+    int rc = track_state_args(state, n_seq, max_tracks, "ekp_smooth_reset");
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    CU(cudaMemsetAsync(state, 0, (size_t) ekp_smooth_state_bytes(n_seq, max_tracks), (cudaStream_t) stream));
+    return EKP_OK;
+}
+
+extern "C" int ekp_smooth_humans(ekp_ctx* c, const int* num_humans, const ekp_peak* parts, const int* ids, int n, int max_humans,
+                                 void* state, int n_seq, int max_tracks, int max_age, double fps, double min_cutoff, double beta,
+                                 double d_cutoff, float* xy, void* stream) {
+    if (!c) return fail(EKP_ERR_ARG, "ekp_smooth_humans: NULL context");
+    int rc = smooth_args_ok(num_humans, parts, ids, n, max_humans, state, n_seq, max_tracks, max_age, fps, min_cutoff, beta, d_cutoff,
+                            xy, "ekp_smooth_humans");
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    CU(launch_smooth(num_humans, parts, ids, n, max_humans, state, n_seq, max_tracks, max_age, fps, min_cutoff, beta, d_cutoff, xy,
+                     (cudaStream_t) stream));
+    c->launches += 1;
+    return EKP_OK;
+}
+
+extern "C" int ekp_debug_smooth_host(const int* num_humans, const ekp_peak* parts, const int* ids, int n, int max_humans, void* state,
+                                     int n_seq, int max_tracks, int max_age, double fps, double min_cutoff, double beta, double d_cutoff,
+                                     float* xy) {
+    int rc = smooth_args_ok(num_humans, parts, ids, n, max_humans, state, n_seq, max_tracks, max_age, fps, min_cutoff, beta, d_cutoff,
+                            xy, "ekp_debug_smooth_host");
+    if (rc) return rc;
+    debug_smooth_host(num_humans, parts, ids, n, max_humans, state, n_seq, max_tracks, max_age, fps, min_cutoff, beta, d_cutoff, xy);
     return EKP_OK;
 }
 

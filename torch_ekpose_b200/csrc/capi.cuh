@@ -52,6 +52,13 @@ cudaError_t launch_track(const int* num_humans, const ekp_peak* parts, int n, in
                          float min_oks, int max_age, int* ids, cudaStream_t stream);
 void debug_track_host(const int* num_humans, const ekp_peak* parts, int n, int max_humans, void* state, int n_seq, int max_tracks,
                       float min_oks, int max_age, int* ids);
+size_t smooth_state_seq_bytes(int max_tracks);
+cudaError_t configure_smooth();
+cudaError_t launch_smooth(const int* num_humans, const ekp_peak* parts, const int* ids, int n, int max_humans, void* state, int n_seq,
+                          int max_tracks, int max_age, double fps, double min_cutoff, double beta, double d_cutoff, float* xy,
+                          cudaStream_t stream);
+void debug_smooth_host(const int* num_humans, const ekp_peak* parts, const int* ids, int n, int max_humans, void* state, int n_seq,
+                       int max_tracks, int max_age, double fps, double min_cutoff, double beta, double d_cutoff, float* xy);
 cudaError_t configure_coco_eval();
 size_t coco_eval_ws_bytes(long long n_img, long long max_det, int A);
 size_t coco_img_smem_bytes(int max_gt, int max_dt, int max_det);

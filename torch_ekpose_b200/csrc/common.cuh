@@ -133,6 +133,16 @@ inline void oks_vars(double var[17]) {
     }
 }
 
+// The track-table rules of a sequence of frames, one copy for the tracker (track.cu) and the smoother (smooth.cu): an
+// entry last seen at frame last_seen is dropped at frame last_seen + max_age + 2, and a new entry that finds no free one
+// takes that of the smallest (last_seen, id) among those not seen in the current frame.
+__host__ __device__ __forceinline__ bool expired(int last_seen, int f, int max_age) {
+    return (long long) f - last_seen > (long long) max_age + 1;
+}
+__host__ __device__ __forceinline__ bool evict_first(int seen_a, int id_a, int seen_b, int id_b) {
+    return seen_a < seen_b || (seen_a == seen_b && id_a < id_b);
+}
+
 // launch parameter blocks --------------------------------------------------------------------
 struct AsmParams {
     const ekp_peak* line;      // [n][max_peaks] part-sorted peak table

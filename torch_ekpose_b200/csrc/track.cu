@@ -131,14 +131,10 @@ HD double oks(const TrackSlot& t, const PersonPose& p, const double* var) {
     return s / m;
 }
 
-// the matching rules: the order of a person's candidate tracks (key: the track's tag, i.e. its id) and of a track's
-// candidate people (key: the row) -- both the total order's restriction to pairs sharing that person or track --,
-// liveness, and the order in which the slots of unmatched live tracks are reused
+// the matching rule: the order of a person's candidate tracks (key: the track's tag, i.e. its id) and of a track's
+// candidate people (key: the row) -- both the total order's restriction to pairs sharing that person or track.
+// Liveness and the order in which the slots of unmatched live tracks are reused are common.cuh's expired / evict_first.
 HD bool pair_first(double sa, int key_a, double sb, int key_b) { return sa > sb || (sa == sb && key_a < key_b); }
-HD bool expired(int last_seen, int f, int max_age) { return (long long) f - last_seen > (long long) max_age + 1; }
-HD bool evict_first(const TrackSlot& a, const TrackSlot& b) {
-    return a.last_seen < b.last_seen || (a.last_seen == b.last_seen && a.tag < b.tag);
-}
 
 struct TrackArgs {
     const int* num_humans;   // [n]
@@ -312,7 +308,7 @@ HD void track_sequence(const TrackArgs& A, int seq, const TrackWork& W, int tid,
                 int r = 0;
                 for (int q = 0; q < L; q++) {
                     const TrackSlot& o = W.slot[W.live[q]];
-                    r += o.last_seen != f && evict_first(o, s);
+                    r += o.last_seen != f && evict_first(o.last_seen, o.tag, s.last_seen, s.tag);  // tags order as ids
                 }
                 if (r < B - Fr) W.freel[Fr + r] = W.live[k];
             }

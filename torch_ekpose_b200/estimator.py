@@ -99,7 +99,7 @@ def infer_humans(images: Sequence[np.ndarray], model, preprocess: str, device, f
 
 
 def infer_human_tensors(images, model, preprocess: str, device, frontend: str = "reference", thr: float = 0.15,
-                        subset: bool = False, peaks: bool = False, tracker=None):
+                        subset: bool = False, peaks: bool = False, tracker=None, smoother=None):
     """``infer_humans`` with the people left on the GPU: returns (tensors, im_scale), ``tensors`` being the dict of
     CUDA tensors ``PostProcessor.result_tensors(subset=subset)`` returns (per image num_humans, overflow, n_peaks,
     the part table, part and human scores; with ``peaks=True`` also the peak table) and ``im_scale`` that of
@@ -107,11 +107,16 @@ def infer_human_tensors(images, model, preprocess: str, device, frontend: str = 
     ``tensors['overflow']``.  The batch leaves its records on the device (no copy to the host); ``last_postprocessor()``'s
     host readers still work, at the cost of one download.  With a ``Tracker`` (``tracking.py``) of the same device,
     ``tensors['track_id']`` (int32 [n, max_humans]) holds each person's id across calls, computed on the export's
-    stream."""
+    stream.  With a ``Smoother`` (``smoothing.py``) as well, ``tensors['smoothed_xy']`` (float32 [n, max_humans, 18, 2])
+    holds the keypoints filtered per track id, on the same stream; a smoother without a tracker is a ValueError."""
+    if smoother is not None and tracker is None:
+        raise ValueError("smoother= needs tracker=: the filters are kept per track id")
     pafs, heats, im_scale = get_outputs_batched(images, model, preprocess, device)
     tensors = _postprocess(heats, pafs, frontend, thr, False).result_tensors(subset=subset, peaks=peaks)
     if tracker is not None:
         tensors["track_id"] = tracker.update(tensors)
+    if smoother is not None:
+        tensors["smoothed_xy"] = smoother.update(tensors, tensors["track_id"])
     return tensors, im_scale
 
 
